@@ -1,12 +1,18 @@
 #!/usr/bin/env python
 """bench.py -- QPS of the Vamana batched search (BASELINE.json metric) on B200, one JSON line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], the configuration the metric is quoted on): synthetic 1M x 96-d
 float32, L2, Vamana search_window=128, batch = 10k queries, k = 10; graph built once per box by the
-reference's own CPU builder (oracle/_ref, R=64, window 128, alpha 1.2) and cached under /tmp.
-A "step" = one full pass of the hot path over the 10k-query batch.
+reference's own CPU builder (oracle/_ref, R=64, window 128, alpha 1.2) and cached in the system's temporary
+directory.  oracle/_ref can only be compiled where the reference's sources are; without it (and without a cached
+graph) the graph comes from the project's GPU builder (svsb200_build_vamana, same parameters), and the line's
+config.graph_builder says which.  A "step" = one full pass of the hot path over the 10k-query batch.
+--dump-outputs DIR writes the results of the last timed step (ids as float64, distances as float32) to
+DIR/ids.npy and DIR/distances.npy.  Data and queries come from fixed seeds and the graph is cached per box, so runs
+with the same arguments search the same inputs and two builds can be compared output for output (a graph built
+afresh can differ in a few edges: both builders' results depend on thread timing).
 
 Lines printed (rank 0 only):
   value     whole-job QPS with queries/results resident in HBM (CUDA events, max over ranks)
@@ -21,6 +27,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -81,13 +88,29 @@ def dist_env():
 
 
 # ------------------------------------------------------------------------------------------------
-# workload: data + graph (cached per box under /tmp, rank 0 builds)
+# workload: data + graph (cached per box in the temporary directory, rank 0 builds)
 # ------------------------------------------------------------------------------------------------
-def build_graph_cached(tag, w, base, rank_builds, barrier):
-    """Vamana graph from the reference's own CPU builder (oracle/_ref), cached per box under /tmp."""
+def graph_cache_path(tag, w):
     key = hashlib.sha1(json.dumps({k: w.get(k) for k in ("n", "dim", "dtype", "metric", "max_degree", "build_window",
                                                            "alpha", "builder")}, sort_keys=True).encode()).hexdigest()[:12]
-    cache = os.path.join(os.environ.get("SVSB200_CACHE", "/tmp/svsb200_cache"), f"graph_{tag}_{key}.npy")
+    return os.path.join(os.environ.get("SVSB200_CACHE") or os.path.join(tempfile.gettempdir(), "svsb200_cache"),
+                        f"graph_{tag}_{key}.npy")
+
+
+def graph_source(tag, w):
+    """`w` with the builder its graph comes from: the reference's CPU builder where oracle/_ref is built or its graph
+    is cached, otherwise the GPU builder (oracle/_ref needs the reference's sources to compile)."""
+    from oracle.bindings import RefLib
+    if w.get("builder") or os.path.exists(graph_cache_path(tag, w)) or RefLib.available():
+        return w
+    log(f"oracle/_ref/libsvsref.so is not built: graph {tag} from the GPU builder (svsb200_build_vamana)")
+    return dict(w, builder="gpu")
+
+
+def build_graph_cached(tag, w, base, rank_builds, barrier):
+    """Vamana graph from the GPU builder or the reference's own CPU builder (oracle/_ref), cached per box in the
+    temporary directory."""
+    cache = graph_cache_path(tag, w)
     if w.get("per_shard_data") and w.get("builder") == "gpu":
         # multi-GB shard graphs: built in place on this rank's GPU, never written to disk
         from scalablevectorsearch_b200 import DistanceType, VamanaBuildParameters, build_graph
@@ -143,7 +166,9 @@ def load_workload(name, rank, world, barrier):
     if w["dtype"] == "float16":
         base = base.astype(np.float16)
     gname = w.get("graph_from", name)
-    ep, graph = build_graph_cached(gname, WORKLOADS[gname], base, rank == 0, barrier)
+    gw = graph_source(gname, WORKLOADS[gname])
+    w = dict(w, builder=gw.get("builder"))
+    ep, graph = build_graph_cached(gname, gw, base, rank == 0, barrier)
     log(f"rank {rank}: workload {name} ready in {time.time() - t0:.1f} s (entry point {ep})")
     return w, base, queries, graph, ep
 
@@ -226,7 +251,9 @@ def run_reference(args):
     threads = effective_cpus()
     # the CPU path's QPS does not depend on how many GPUs our arm uses: each step is one 10k-query batch of the
     # same workload (a bounded sample of the N x 10k global batch of the weak-scaling run)
-    times, _, _, ref = time_reference(w, base, queries, graph, ep, args.steps, args.warmup, threads)
+    times, ids, dists, ref = time_reference(w, base, queries, graph, ep, args.steps, args.warmup, threads)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ids=ids, distances=dists)
     total = sum(times)
     qps = w["nq"] * len(times) / total
     line = {
@@ -247,6 +274,15 @@ REF_PAGES = ("reference data+graph in lib::Allocator memory = 4 KiB pages (trans
              "setting); its HugepageAllocator (core/allocator.h:94-150) is not used by this arm")
 
 
+def dump_outputs(directory, **arrays):
+    """Save each result array of the last timed step as DIR/<name>.npy: integer ids as float64 (exact below 2^53),
+    distances as float32."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if hasattr(a, "cpu") else np.asarray(a)
+        np.save(os.path.join(directory, f"{name}.npy"), a.astype(np.float64 if a.dtype.kind in "iu" else np.float32))
+
+
 def run_config(name, w, graph, gpus, weak):
     """The `config` object, identical in both arms (the driver compares them)."""
     return dict(workload_config(name, w, graph), global_batch=w["nq"] * (gpus if weak else 1),
@@ -256,7 +292,7 @@ def run_config(name, w, graph, gpus, weak):
 def workload_config(name, w, graph):
     return {"workload": name, "n": w["n"], "dim": w["dim"], "base_dtype": w["dtype"], "distance": w["metric"],
             "batch": w["nq"], "k": w["k"], "search_window": w["window"], "graph_max_degree": w["max_degree"],
-            "graph_avg_degree": round(float(graph[:, 0].mean()), 2),
+            "graph_avg_degree": round(float(graph[:, 0].mean()), 2), "graph_builder": w.get("builder") or "reference cpu",
             "l2_policy": "index (vectors+graph) is several times larger than the 126 MB L2; no explicit flush"}
 
 
@@ -337,6 +373,7 @@ def run_ours(args):
         stop.record()
         torch.cuda.synchronize()
         launched = lib.svsb200_launch_count() - l0
+        out = tuple(t.clone() for t in out)   # the multi-GPU gather reuses its buffers on the next call
         barrier()
         ms = start.elapsed_time(stop)
         kern = []
@@ -366,6 +403,8 @@ def run_ours(args):
 
     with ClockSampler(local_rank) as clocks:
         elapsed_ms, kern_ms, (ids_all, d_all), q_dev, launches = time_mode(q_strong)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ids=ids_all, distances=d_all)
     qps = nq * args.steps / (elapsed_ms * 1e-3)
     weak = None
     if world > 1:
@@ -636,6 +675,8 @@ def run_sharded(args):
     else:
         parts, gts = [(r_ids, r_d)], [(gt_i.cpu().numpy() + lo, gt_d.cpu().numpy())]
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, ids=ids, distances=d)
         gt_ids, _ = merge_topk_reference_order(np.stack([g_[0] for g_ in gts]), np.stack([g_[1] for g_ in gts]), k,
                                                w["metric"] != "l2")
         got = ids[:ns].cpu().numpy()
@@ -683,7 +724,11 @@ def main():
                          "result as `value` and the weak one under `weak` in the same line)")
     ap.add_argument("--cpu-sample", dest="cpu_sample", type=int, default=0,
                     help="cpu_baseline: time only the first N queries of the batch (bounded sample for big workloads)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", default=None, metavar="DIR",
+                    help="write the results of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if WORKLOADS[args.workload].get("sharded"):
         run_sharded(args)
     elif args.impl == "reference":

@@ -56,6 +56,12 @@ def ref_outputs():
 
 
 @pytest.fixture(scope="session")
+def ref_checks():
+    """What the compiled reference computed for the oracle and graph-builder tests (tests/golden/make_golden.py)."""
+    return np.load(os.path.join(GOLDEN, "ref_checks.npz"))
+
+
+@pytest.fixture(scope="session")
 def golden_recalls():
     return json.load(open(os.path.join(GOLDEN, "golden_recalls.json")))
 

@@ -7,6 +7,8 @@ Outputs: test_dataset.npz   compact copy of the fixtures the parity tests need o
          ref_outputs.npz    ids / distances / work counters the *reference itself* produces
          golden_recalls.json the 17 (window, capacity) -> recall@10 goldens of
                             data/test_dataset/reference/vamana_reference.toml (vamana_test_search)
+         ref_checks.npz     the reference on random non-integer inputs and its CPU graph builder's results
+                            (write_ref_checks)
 
     python tests/golden/make_golden.py
 """
@@ -105,6 +107,54 @@ def main():
     np.savez_compressed(f"{OUT}/ref_outputs.npz", **outs)
     for f in ("test_dataset.npz", "ref_outputs.npz", "golden_recalls.json"):
         print(f, os.path.getsize(f"{OUT}/{f}") // 1024, "KiB")
+    write_ref_checks(ref)
+
+
+def write_ref_checks(ref):
+    """ref_checks.npz: what the reference computes for tests/test_oracle_golden.py (distances and searches on
+    random non-integer inputs, stored with them) and tests/test_gpu_build.py (its CPU builder's entry point, average
+    degree and the recall@10 of its graphs, searched by the oracle, which is bit-identical to the GPU search)."""
+    from oracle.bindings import OracleLib
+    from scalablevectorsearch_b200.synthetic import clustered_unit_vectors
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from conftest import Dataset, knn_graph, recall_at_k
+
+    out = {}
+    rng = np.random.default_rng(11)
+    for dim in (17, 96, 100, 768):
+        q = rng.standard_normal(dim).astype(np.float32)
+        x = rng.standard_normal((40, dim)).astype(np.float32)
+        out[f"live_q_{dim}"], out[f"live_x_{dim}"] = q, x
+        for metric in ("l2", "ip", "cosine"):
+            for p, (qq, xx) in enumerate(((q, x), (q, x.astype(np.float16)), (q.astype(np.float16), x.astype(np.float16)))):
+                out[f"live_dist_{dim}_{metric}_{p}"] = ref.distance_rows(metric, qq, xx)
+    n, dim = 1200, 48
+    x = rng.standard_normal((n, dim)).astype(np.float32)
+    qs = rng.standard_normal((100, dim)).astype(np.float32)
+    graph = knn_graph(x, 12, rng)
+    out["live_x"], out["live_queries"], out["live_graph"] = x, qs, graph
+    for metric in ("l2", "ip", "cosine"):
+        ids, dists = ref.index(x, graph, 5, metric).search(qs, 5, 9, 14)
+        out[f"live_{metric}_ids"], out[f"live_{metric}_dists"] = ids.astype(np.uint32), dists
+
+    oracle, ds = OracleLib(), Dataset()
+    for metric in ("l2", "ip", "cosine"):
+        g, ep = ref.build(ds.data, metric, 32, 64, alpha=1.2 if metric == "l2" else 0.95, threads=4)
+        idx = oracle.index(ds.data, g, ep, metric)
+        out[f"build_{metric}_entry_point"] = np.uint32(ep)
+        out[f"build_{metric}_avg_degree"] = np.float64(g[:, 0].mean())
+        out[f"build_{metric}_recall_w10_w30"] = np.array(
+            [recall_at_k(idx.search(ds.queries, 10, w, w)[0], ds.gt[metric]) for w in (10, 30)])
+    base, queries = clustered_unit_vectors(30_000, 500, 96)
+    base16 = base.astype(np.float16)
+    xf = base16.astype(np.float32)
+    d = (queries ** 2).sum(1)[:, None] + (xf ** 2).sum(1)[None, :] - 2.0 * queries @ xf.T
+    gt = np.argsort(d, axis=1, kind="stable")[:, :10]
+    g, ep = ref.build(base16, "l2", 64, 128, alpha=1.2, threads=8)
+    out["build_synthetic_f16_recall_w64"] = np.float64(
+        recall_at_k(oracle.index(base16, g, ep, "l2").search(queries, 10, 64, 64)[0], gt))
+    np.savez_compressed(f"{OUT}/ref_checks.npz", **out)
+    print("ref_checks.npz", os.path.getsize(f"{OUT}/ref_checks.npz") // 1024, "KiB")
 
 
 if __name__ == "__main__":

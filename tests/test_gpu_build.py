@@ -3,8 +3,8 @@
 The reference's build result depends on thread timing, so its own tests compare recall, not graphs
 (tests/integration/vamana/index_build.cpp:96,139-140: |recall - expected| < 0.005 between runs of the same builder).
 Here: same data, same parameters, the graph from the GPU builder vs the graph from the reference's CPU builder
-(oracle/_ref), both searched by the bit-exact GPU search; recall@10 must agree within 0.01 and the graphs must have a
-similar density.  Structural checks: degrees within bounds, no self loops, no repeated neighbours, ids in range."""
+(its entry point, average degree and recall@10 under the bit-exact search, stored in tests/golden/ref_checks.npz);
+recall@10 must agree within 0.01 and the graphs must have a similar density.  Structural checks: degrees within bounds, no self loops, no repeated neighbours, ids in range."""
 import numpy as np
 import pytest
 
@@ -30,7 +30,7 @@ def _recall(data, graph, ep, queries, gt, metric, window):
 
 
 @pytest.mark.parametrize("metric", ["l2", "ip", "cosine"])
-def test_build_on_reference_dataset_matches_reference_builder_recall(dataset, reflib, metric):
+def test_build_on_reference_dataset_matches_reference_builder_recall(dataset, ref_checks, metric):
     """data/test_dataset (10k x 128), the reference's own build test shape (index_build.cpp: R=64... here R=32,
     window 64 to keep the CPU side quick)."""
     from scalablevectorsearch_b200 import DistanceType, VamanaBuildParameters, build_graph
@@ -39,18 +39,17 @@ def test_build_on_reference_dataset_matches_reference_builder_recall(dataset, re
     params = VamanaBuildParameters(alpha=alpha, graph_max_degree=32, window_size=64)
     g_gpu, ep_gpu = build_graph(dataset.data, dist, params)
     _structural(g_gpu, dataset.data.shape[0], 32)
-    g_ref, ep_ref = reflib.build(dataset.data, metric, 32, 64, alpha=alpha, threads=4)
+    ep_ref = int(ref_checks[f"build_{metric}_entry_point"])
     assert ep_gpu == ep_ref, "medoid entry point differs from the reference's"
     q, gt = dataset.queries, dataset.gt[metric]
-    for window in (10, 30):
+    for window, r_ref in zip((10, 30), ref_checks[f"build_{metric}_recall_w10_w30"]):
         r_gpu = _recall(dataset.data, g_gpu, ep_gpu, q, gt, metric, window)
-        r_ref = _recall(dataset.data, g_ref, ep_ref, q, gt, metric, window)
         assert r_gpu >= r_ref - 0.01, (metric, window, r_gpu, r_ref)
-    d_gpu, d_ref = g_gpu[:, 0].mean(), g_ref[:, 0].mean()
+    d_gpu, d_ref = g_gpu[:, 0].mean(), float(ref_checks[f"build_{metric}_avg_degree"])
     assert 0.8 * d_ref <= d_gpu <= 1.25 * d_ref, (d_gpu, d_ref)
 
 
-def test_build_synthetic_f16_and_index_build_api(reflib):
+def test_build_synthetic_f16_and_index_build_api(ref_checks):
     """Clustered unit vectors (the bench's law), float16 storage, through Vamana.build; recall vs brute force."""
     from scalablevectorsearch_b200 import DistanceType, SearchBufferConfig, Vamana, VamanaBuildParameters
     from scalablevectorsearch_b200.synthetic import clustered_unit_vectors
@@ -62,8 +61,6 @@ def test_build_synthetic_f16_and_index_build_api(reflib):
     x = base16.astype(np.float32)
     d = (queries ** 2).sum(1)[:, None] + (x ** 2).sum(1)[None, :] - 2.0 * queries @ x.T
     gt = np.argsort(d, axis=1, kind="stable")[:, :10]
-    g_ref, ep_ref = reflib.build(base16, "l2", 64, 128, alpha=1.2, threads=8)
-    ref_index = Vamana.from_arrays(base16, g_ref, ep_ref, DistanceType.L2)
-    ref_index.search_parameters.buffer_config = SearchBufferConfig(64)
-    r_gpu, r_ref = recall_at_k(ids, gt), recall_at_k(ref_index.search(queries, 10)[0], gt)
+    # the reference's CPU builder (R 64, window 128, alpha 1.2) on the same data, searched at window 64
+    r_gpu, r_ref = recall_at_k(ids, gt), float(ref_checks["build_synthetic_f16_recall_w64"])
     assert r_gpu >= r_ref - 0.01 and r_gpu > 0.9, (r_gpu, r_ref)

@@ -1,10 +1,10 @@
 """Pin the oracle: the plain-C restatement vs (a) the reference's 17 golden recalls, (b) the committed
-outputs of the reference itself, (c) the compiled reference live (when oracle/_ref loads here),
+outputs of the reference itself, (c) the compiled reference on random non-integer inputs (stored outputs),
 (d) a double-precision model with the reference's own tolerance."""
 import numpy as np
 import pytest
 
-from conftest import bits, knn_graph, recall_at_k
+from conftest import bits, recall_at_k
 
 
 @pytest.mark.parametrize("metric", ["l2", "ip", "cosine"])
@@ -71,22 +71,19 @@ def test_oracle_distances_vs_double_precision(oracle):
                 assert np.all(np.abs(got - w) <= eps * np.maximum(scale, 1e-30) * 4), (dim, qd, xd, metric)
 
 
-def test_oracle_matches_compiled_reference_live(oracle, reflib):
-    """Bit-exact distances and searches against oracle/_ref on fresh random inputs (non-integer data)."""
-    rng = np.random.default_rng(11)
+def test_oracle_matches_compiled_reference_live(oracle, ref_checks):
+    """Bit-exact distances and searches against the compiled reference on random non-integer inputs (inputs and
+    the reference's outputs stored in tests/golden/ref_checks.npz by tests/golden/make_golden.py)."""
     for dim in (17, 96, 100, 768):
-        q = rng.standard_normal(dim).astype(np.float32)
-        x = rng.standard_normal((40, dim)).astype(np.float32)
+        q, x = ref_checks[f"live_q_{dim}"], ref_checks[f"live_x_{dim}"]
         for metric in ("l2", "ip", "cosine"):
-            for qq, xx in ((q, x), (q, x.astype(np.float16)), (q.astype(np.float16), x.astype(np.float16))):
-                assert np.array_equal(bits(oracle.distance_rows(metric, qq, xx)), bits(reflib.distance_rows(metric, qq, xx)))
-    n, dim = 1200, 48
-    x = rng.standard_normal((n, dim)).astype(np.float32)
-    qs = rng.standard_normal((100, dim)).astype(np.float32)
-    graph = knn_graph(x, 12, rng)
+            for p, (qq, xx) in enumerate(((q, x), (q, x.astype(np.float16)), (q.astype(np.float16), x.astype(np.float16)))):
+                want = ref_checks[f"live_dist_{dim}_{metric}_{p}"]
+                assert np.array_equal(bits(oracle.distance_rows(metric, qq, xx)), bits(want)), (dim, metric, p)
+    x, qs, graph = ref_checks["live_x"], ref_checks["live_queries"], ref_checks["live_graph"]
     for metric in ("l2", "ip", "cosine"):
+        b = ref_checks[f"live_{metric}_ids"].astype(np.uint64), ref_checks[f"live_{metric}_dists"]
         a = oracle.index(x, graph, 5, metric).search(qs, 5, 9, 14)
-        b = reflib.index(x, graph, 5, metric).search(qs, 5, 9, 14)
         assert np.array_equal(a[0], b[0]) and np.array_equal(bits(a[1]), bits(b[1]))
         a = oracle.index(x, graph, 5, metric).search(qs, 5, 9, 14, visited_set=True)
         assert np.array_equal(a[0], b[0]) and np.array_equal(bits(a[1]), bits(b[1]))
