@@ -7,15 +7,6 @@
 
 namespace svsb200 {
 
-#define BUILD_TRY(expr)                                                                        \
-    do {                                                                                       \
-        cudaError_t err__ = (expr);                                                            \
-        if (err__ != cudaSuccess) {                                                            \
-            rc = set_error(std::string(#expr) + ": " + cudaGetErrorString(err__));             \
-            goto done;                                                                         \
-        }                                                                                      \
-    } while (0)
-
 // add_reverse_edges, first half (vamana_build.h:484-501): one thread per new edge v -> u.
 __global__ void reverse_insert_kernel(uint32_t first, uint32_t count, uint32_t* __restrict__ graph, uint32_t* __restrict__ deg,
                                       uint32_t gstride, uint32_t max_degree, int* __restrict__ head, int* __restrict__ next,
@@ -173,214 +164,195 @@ extern "C" int svsb200_build_vamana(const void* vectors, int dtype, size_t n, si
     if (alpha == 0.f) alpha = metric == SVSB200_L2 ? 1.2f : 0.95f;
     if (metric == SVSB200_L2 ? alpha < 1.0f : alpha > 1.0f) return set_error("svsb200_build_vamana: alpha on the wrong side of 1 for this metric");
     const uint32_t R = uint32_t(graph_max_degree);
-    const uint32_t gstride = (R + 31u) & ~31u;
+    const uint32_t gstride = gstride_for(R);
     const uint32_t hist_cap = kPoolMax - gstride;
     if (window_size + 32 > hist_cap) return set_error("svsb200_build_vamana: window_size too large for the candidate pool");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return set_error("svsb200_build_vamana: no CUDA device (there is no CPU fallback)");
-    }
+    const int ndev = svsb200_device_count();
+    if (ndev == 0) return set_error("svsb200_build_vamana: no CUDA device (there is no CPU fallback)");
     if (device < 0 || device >= ndev) return set_error("svsb200_build_vamana: bad device ordinal");
     cudaDeviceProp prop;
     if (cudaSetDevice(device) != cudaSuccess || cudaGetDeviceProperties(&prop, device) != cudaSuccess)
         return set_error("svsb200_build_vamana: cannot select the device");
     if (prop.major != 10 || prop.minor != 0) return set_error("svsb200_build_vamana: device is not sm_100");
 
-    const size_t es = dtype == SVSB200_F32 ? 4 : 2;
-    const size_t row_bytes = dim * es;
+    const size_t row_bytes = dim * esize(dtype);
     const size_t src_stride = row_stride_bytes ? row_stride_bytes : row_bytes;
-    const uint32_t row_stride = uint32_t((row_bytes + 15) / 16 * 16);
-    const uint32_t qstride = uint32_t((dim + 15) / 16 * 16);
+    const uint32_t row_stride = row_stride_for(SVSB200_PLAIN, dtype, dim);
+    const uint32_t qstride = qstride_for(dim);
     // batches (vamana_build.h:229-240)
     size_t num_batches = std::max<size_t>(40, (n + 4095) / 4096);
     if (num_batches > n) num_batches = n;
     const size_t batchsize = (n + num_batches - 1) / num_batches;
-
-    int rc = 0;
-    char* d_vectors = nullptr;
-    uint32_t *d_graph = nullptr, *d_deg = nullptr, *d_hist_count = nullptr, *d_pair_v = nullptr, *d_counts = nullptr,
-             *d_touched = nullptr, *d_best_i = nullptr, *d_export = nullptr;
-    int *d_head = nullptr, *d_next = nullptr;
-    uint2* d_hist = nullptr;
-    float *d_qf = nullptr, *d_qaux = nullptr;
-    double *d_sums = nullptr, *d_best_d = nullptr;
-    unsigned int* d_work = nullptr;
-    cudaStream_t stream = nullptr;
     const size_t pair_cap = batchsize * R;
     const int grid_sm = prop.multiProcessorCount;
+    const unsigned nblk = unsigned((n + 7) / 8);   // blocks of the medoid search
+
+    cudaStream_t stream = nullptr;
+    CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+    StreamOwner stream_owner(stream, cudaStreamDestroy);   // (declared first: destroyed after every buffer is freed)
+    DeviceBuffer<char> d_vectors;
+    DeviceBuffer<uint32_t> d_graph, d_deg, d_hist_count, d_pair_v, d_counts, d_touched, d_best_i, d_export;
+    DeviceBuffer<int> d_head, d_next;
+    DeviceBuffer<uint2> d_hist;
+    DeviceBuffer<float> d_qf, d_qaux;
+    DeviceBuffer<double> d_sums, d_best_d;
+    DeviceBuffer<unsigned int> d_work;
+    CUDA_TRY(d_vectors.ensure(n * size_t(row_stride)));
+    CUDA_TRY(cudaMemset(d_vectors.ptr, 0, n * size_t(row_stride)));
+    CUDA_TRY(cudaMemcpy2D(d_vectors.ptr, row_stride, vectors, src_stride, row_bytes, n, cudaMemcpyHostToDevice));
+    CUDA_TRY(d_graph.ensure(n * size_t(gstride)));
+    CUDA_TRY(d_deg.ensure(n));
+    CUDA_TRY(cudaMemset(d_deg.ptr, 0, n * 4));
+    CUDA_TRY(d_head.ensure(n));
+    CUDA_TRY(cudaMemset(d_head.ptr, 0xFF, n * 4));
+    CUDA_TRY(d_next.ensure(pair_cap));
+    CUDA_TRY(d_pair_v.ensure(pair_cap));
+    CUDA_TRY(d_touched.ensure(pair_cap));
+    CUDA_TRY(d_counts.ensure(2));
+    CUDA_TRY(d_hist.ensure(batchsize * size_t(hist_cap)));
+    CUDA_TRY(d_hist_count.ensure(batchsize));
+    CUDA_TRY(d_qf.ensure(batchsize * size_t(qstride)));
+    CUDA_TRY(d_qaux.ensure(batchsize * 2));
+    CUDA_TRY(cudaMemset(d_qaux.ptr, 0, batchsize * 2 * 4));
+    CUDA_TRY(d_work.ensure(1));
+    CUDA_TRY(d_sums.ensure(dim));
+    CUDA_TRY(cudaMemset(d_sums.ptr, 0, dim * 8));
+    {
+        const size_t cnt = n * size_t(gstride);
+        fill_u32_kernel<<<unsigned((cnt + 255) / 256), 256, 0, stream>>>(d_graph.ptr, cnt, kNoNeighbor);
+        count_launch();
+    }
+    // ---- entry point = medoid (index.h:986-990, core/medioid.h:292-330) ----
     uint32_t entry_point = 0;
     {
-        BUILD_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-        BUILD_TRY(cudaMalloc(&d_vectors, n * size_t(row_stride)));
-        BUILD_TRY(cudaMemset(d_vectors, 0, n * size_t(row_stride)));
-        BUILD_TRY(cudaMemcpy2D(d_vectors, row_stride, vectors, src_stride, row_bytes, n, cudaMemcpyHostToDevice));
-        BUILD_TRY(cudaMalloc(&d_graph, n * size_t(gstride) * 4));
-        BUILD_TRY(cudaMalloc(&d_deg, n * 4));
-        BUILD_TRY(cudaMemset(d_deg, 0, n * 4));
-        BUILD_TRY(cudaMalloc(&d_head, n * 4));
-        BUILD_TRY(cudaMemset(d_head, 0xFF, n * 4));
-        BUILD_TRY(cudaMalloc(&d_next, pair_cap * 4));
-        BUILD_TRY(cudaMalloc(&d_pair_v, pair_cap * 4));
-        BUILD_TRY(cudaMalloc(&d_touched, pair_cap * 4));
-        BUILD_TRY(cudaMalloc(&d_counts, 2 * 4));
-        BUILD_TRY(cudaMalloc(&d_hist, batchsize * size_t(hist_cap) * 8));
-        BUILD_TRY(cudaMalloc(&d_hist_count, batchsize * 4));
-        BUILD_TRY(cudaMalloc(&d_qf, batchsize * size_t(qstride) * 4));
-        BUILD_TRY(cudaMalloc(&d_qaux, batchsize * 2 * 4));
-        BUILD_TRY(cudaMemset(d_qaux, 0, batchsize * 2 * 4));
-        BUILD_TRY(cudaMalloc(&d_work, 4));
-        BUILD_TRY(cudaMalloc(&d_sums, dim * 8));
-        BUILD_TRY(cudaMemset(d_sums, 0, dim * 8));
-        {
-            const size_t cnt = n * size_t(gstride);
-            fill_u32_kernel<<<unsigned((cnt + 255) / 256), 256, 0, stream>>>(d_graph, cnt, kNoNeighbor);
-            count_launch();
+        CUDA_TRY(d_best_d.ensure(nblk));
+        CUDA_TRY(d_best_i.ensure(nblk));
+        if (dtype == SVSB200_F32) {
+            column_sum_kernel<SVSB200_F32><<<unsigned((n + 255) / 256), 128, 0, stream>>>(d_vectors.ptr, uint32_t(n), uint32_t(dim), row_stride, d_sums.ptr);
+            medoid_distance_kernel<SVSB200_F32><<<nblk, 256, 0, stream>>>(d_vectors.ptr, uint32_t(n), uint32_t(dim), row_stride, d_sums.ptr, d_best_d.ptr, d_best_i.ptr);
+        } else {
+            column_sum_kernel<SVSB200_F16><<<unsigned((n + 255) / 256), 128, 0, stream>>>(d_vectors.ptr, uint32_t(n), uint32_t(dim), row_stride, d_sums.ptr);
+            medoid_distance_kernel<SVSB200_F16><<<nblk, 256, 0, stream>>>(d_vectors.ptr, uint32_t(n), uint32_t(dim), row_stride, d_sums.ptr, d_best_d.ptr, d_best_i.ptr);
         }
-        // ---- entry point = medoid (index.h:986-990, core/medioid.h:292-330) ----
-        {
-            const unsigned nblk = unsigned((n + 7) / 8);
-            BUILD_TRY(cudaMalloc(&d_best_d, size_t(nblk) * 8));
-            BUILD_TRY(cudaMalloc(&d_best_i, size_t(nblk) * 4));
-            if (dtype == SVSB200_F32) {
-                column_sum_kernel<SVSB200_F32><<<unsigned((n + 255) / 256), 128, 0, stream>>>(d_vectors, uint32_t(n), uint32_t(dim), row_stride, d_sums);
-                medoid_distance_kernel<SVSB200_F32><<<nblk, 256, 0, stream>>>(d_vectors, uint32_t(n), uint32_t(dim), row_stride, d_sums, d_best_d, d_best_i);
-            } else {
-                column_sum_kernel<SVSB200_F16><<<unsigned((n + 255) / 256), 128, 0, stream>>>(d_vectors, uint32_t(n), uint32_t(dim), row_stride, d_sums);
-                medoid_distance_kernel<SVSB200_F16><<<nblk, 256, 0, stream>>>(d_vectors, uint32_t(n), uint32_t(dim), row_stride, d_sums, d_best_d, d_best_i);
-            }
-            count_launch();
-            count_launch();
-            BUILD_TRY(cudaGetLastError());
-            std::vector<double> bd(nblk);
-            std::vector<uint32_t> bi(nblk);
-            BUILD_TRY(cudaMemcpyAsync(bd.data(), d_best_d, size_t(nblk) * 8, cudaMemcpyDeviceToHost, stream));
-            BUILD_TRY(cudaMemcpyAsync(bi.data(), d_best_i, size_t(nblk) * 4, cudaMemcpyDeviceToHost, stream));
-            BUILD_TRY(cudaStreamSynchronize(stream));
-            size_t best = 0;
-            for (size_t b = 1; b < nblk; ++b)
-                if (bd[b] < bd[best]) best = b;
-            entry_point = bi[best];
-        }
-
-        SearchParams p{};
-        p.vectors = d_vectors;
-        p.graph = d_graph;
-        p.ref_degree = nullptr;
-        p.n = uint32_t(n);
-        p.dim = uint32_t(dim);
-        p.row_stride = row_stride;
-        p.gstride = gstride;
-        p.entry_point = entry_point;
-        p.greater = metric != SVSB200_L2;
-        p.scale = 1.f;
-        p.qf = d_qf;
-        p.qcodes = nullptr;
-        p.qaux = d_qaux;
-        p.qstride = qstride;
-        p.k = 0;
-        p.window = uint32_t(window_size);
-        p.capacity = uint32_t(window_size);
-        p.cap_pad = uint32_t((window_size + 31) / 32 * 32);
-        p.deg_pad = gstride;
-        p.id_bytes = 4;
-        p.work_counter = d_work;
-        p.hist = d_hist;
-        p.hist_count = d_hist_count;
-        p.hist_cap = hist_cap;
-        // visited filter of the lean kernel: sets of eight 16-bit tags, enough sets for exact tags
-        uint32_t fslots = 2048, fshift = 8;
-        while ((uint64_t(n - 1) >> fshift) >= 0xFFFFull) {
-            ++fshift;
-            fslots <<= 1;
-        }
-        p.filter_slots = fslots;
-        p.filter_shift = fshift;
-        p.filter_tag16 = 1;
-        LaunchConfig cfg{};
-        cfg.warps_per_cta = 1;
-        cfg.smem_bytes = fast_smem_bytes(qstride, p.cap_pad, p.deg_pad, fslots * 2u);
-        cfg.stream = stream;
-        cfg.grid = -grid_sm;
-        if (cfg.smem_bytes > 227 * 1024) {
-            rc = set_error("svsb200_build_vamana: window_size too large for shared memory");
-            goto done;
-        }
-        const int op = metric == SVSB200_L2 ? OP_L2F : metric == SVSB200_IP ? OP_IPF : OP_COSF;
-
-        BuildParams bp{};
-        bp.hist = d_hist;
-        bp.hist_count = d_hist_count;
-        bp.hist_cap = hist_cap;
-        bp.head = d_head;
-        bp.next = d_next;
-        bp.pair_v = d_pair_v;
-        bp.graph = d_graph;
-        bp.deg = d_deg;
-        bp.gstride = gstride;
-        bp.max_degree = R;
-        bp.max_candidates = uint32_t(std::min<size_t>(max_candidate_pool_size, kPoolMax));
-        bp.iterative = metric != SVSB200_L2;
-        bp.work_counter = d_work;
-        bp.count_ptr = d_counts + 1;
-        bp.nodes = d_touched;
-        const int prune_grid = grid_sm * 16;
-
-        // ---- two passes (index.h:436-439): reverse pruning with alpha 1, then with the configured alpha ----
-        for (int pass = 0; pass < 2; ++pass) {
-            const float reverse_alpha = pass == 0 ? 1.0f : alpha;
-            for (size_t b = 0; b < num_batches; ++b) {
-                const size_t start = std::min(n, batchsize * b), stop = std::min(n, batchsize * (b + 1));
-                if (stop == start) continue;
-                const uint32_t B = uint32_t(stop - start);
-                // 1. generate_neighbors: search ...
-                if (dtype == SVSB200_F32)
-                    batch_queries_kernel<SVSB200_F32><<<(B + 7) / 8, 256, 0, stream>>>(d_vectors, row_stride, uint32_t(dim), qstride, uint32_t(start), B, d_qf, d_qaux);
-                else
-                    batch_queries_kernel<SVSB200_F16><<<(B + 7) / 8, 256, 0, stream>>>(d_vectors, row_stride, uint32_t(dim), qstride, uint32_t(start), B, d_qf, d_qaux);
-                count_launch();
-                BUILD_TRY(cudaMemsetAsync(d_work, 0, 4, stream));
-                p.nq = B;
-                BUILD_TRY(dtype == SVSB200_F32 ? launch_build_search<SVSB200_F32>(op, p, cfg) : launch_build_search<SVSB200_F16>(op, p, cfg));
-                // ... pool + prune (always with the configured alpha, vamana_build.h:268-272)
-                BUILD_TRY(cudaMemsetAsync(d_work, 0, 4, stream));
-                bp.reverse = 0;
-                bp.first = uint32_t(start);
-                bp.count = B;
-                bp.limit = R;
-                bp.alpha = alpha;
-                BUILD_TRY(dtype == SVSB200_F32 ? launch_build_prune_op<SVSB200_F32>(op, p, bp, std::min<int>(prune_grid, int(B)), stream)
-                                               : launch_build_prune_op<SVSB200_F16>(op, p, bp, std::min<int>(prune_grid, int(B)), stream));
-                // 2. add_reverse_edges
-                BUILD_TRY(cudaMemsetAsync(d_counts, 0, 8, stream));
-                reverse_insert_kernel<<<unsigned((size_t(B) * R + 255) / 256), 256, 0, stream>>>(
-                    uint32_t(start), B, d_graph, d_deg, gstride, R, d_head, d_next, d_pair_v, d_counts, d_touched, d_counts + 1,
-                    uint32_t(pair_cap));
-                count_launch();
-                BUILD_TRY(cudaMemsetAsync(d_work, 0, 4, stream));
-                bp.reverse = 1;
-                bp.limit = uint32_t(prune_to);
-                bp.alpha = reverse_alpha;
-                BUILD_TRY(dtype == SVSB200_F32 ? launch_build_prune_op<SVSB200_F32>(op, p, bp, prune_grid, stream)
-                                               : launch_build_prune_op<SVSB200_F16>(op, p, bp, prune_grid, stream));
-                reset_heads_kernel<<<unsigned((pair_cap + 255) / 256), 256, 0, stream>>>(d_touched, d_counts + 1, d_head);
-                count_launch();
-                BUILD_TRY(cudaGetLastError());
-            }
-        }
-        // ---- export in the reference's layout ----
-        BUILD_TRY(cudaMalloc(&d_export, n * size_t(R + 1) * 4));
-        export_graph_kernel<<<unsigned((n + 7) / 8), 256, 0, stream>>>(d_graph, d_deg, uint32_t(n), gstride, R, d_export);
         count_launch();
-        BUILD_TRY(cudaGetLastError());
-        BUILD_TRY(cudaMemcpyAsync(graph_rows_out, d_export, n * size_t(R + 1) * 4, cudaMemcpyDeviceToHost, stream));
-        BUILD_TRY(cudaStreamSynchronize(stream));
-        *entry_point_out = entry_point;
+        count_launch();
+        CUDA_TRY(cudaGetLastError());
+        std::vector<double> bd(nblk);
+        std::vector<uint32_t> bi(nblk);
+        CUDA_TRY(cudaMemcpyAsync(bd.data(), d_best_d.ptr, size_t(nblk) * 8, cudaMemcpyDeviceToHost, stream));
+        CUDA_TRY(cudaMemcpyAsync(bi.data(), d_best_i.ptr, size_t(nblk) * 4, cudaMemcpyDeviceToHost, stream));
+        CUDA_TRY(cudaStreamSynchronize(stream));
+        size_t best = 0;
+        for (size_t b = 1; b < nblk; ++b)
+            if (bd[b] < bd[best]) best = b;
+        entry_point = bi[best];
     }
-done:
-    cudaFree(d_vectors); cudaFree(d_graph); cudaFree(d_deg); cudaFree(d_head); cudaFree(d_next); cudaFree(d_pair_v);
-    cudaFree(d_touched); cudaFree(d_counts); cudaFree(d_hist); cudaFree(d_hist_count); cudaFree(d_qf); cudaFree(d_qaux);
-    cudaFree(d_work); cudaFree(d_sums); cudaFree(d_best_d); cudaFree(d_best_i); cudaFree(d_export);
-    if (stream) cudaStreamDestroy(stream);
-    return rc;
+
+    SearchParams p{};
+    p.vectors = d_vectors.ptr;
+    p.graph = d_graph.ptr;
+    p.ref_degree = nullptr;
+    p.n = uint32_t(n);
+    p.dim = uint32_t(dim);
+    p.row_stride = row_stride;
+    p.gstride = gstride;
+    p.entry_point = entry_point;
+    p.greater = metric != SVSB200_L2;
+    p.scale = 1.f;
+    p.qf = d_qf.ptr;
+    p.qcodes = nullptr;
+    p.qaux = d_qaux.ptr;
+    p.qstride = qstride;
+    p.k = 0;
+    p.window = uint32_t(window_size);
+    p.capacity = uint32_t(window_size);
+    p.cap_pad = uint32_t(round_up(window_size, 32));
+    p.deg_pad = gstride;
+    p.id_bytes = 4;
+    p.work_counter = d_work.ptr;
+    p.hist = d_hist.ptr;
+    p.hist_count = d_hist_count.ptr;
+    p.hist_cap = hist_cap;
+    // visited filter of the lean kernel at its default size, grown as n needs for exact tags
+    const LeanFilterPlan filter = lean_filter_plan(n, dim, window_size, p.deg_pad, 2048);
+    p.filter_slots = filter.slots;
+    p.filter_shift = filter.shift;
+    p.filter_tag16 = 1;
+    LaunchConfig cfg{};
+    cfg.warps_per_cta = 1;
+    cfg.smem_bytes = filter.smem_bytes;
+    cfg.stream = stream;
+    cfg.grid = -grid_sm;
+    if (cfg.smem_bytes > 227 * 1024) return set_error("svsb200_build_vamana: window_size too large for shared memory");
+    const int op = metric == SVSB200_L2 ? OP_L2F : metric == SVSB200_IP ? OP_IPF : OP_COSF;
+
+    BuildParams bp{};
+    bp.hist = d_hist.ptr;
+    bp.hist_count = d_hist_count.ptr;
+    bp.hist_cap = hist_cap;
+    bp.head = d_head.ptr;
+    bp.next = d_next.ptr;
+    bp.pair_v = d_pair_v.ptr;
+    bp.graph = d_graph.ptr;
+    bp.deg = d_deg.ptr;
+    bp.gstride = gstride;
+    bp.max_degree = R;
+    bp.max_candidates = uint32_t(std::min<size_t>(max_candidate_pool_size, kPoolMax));
+    bp.iterative = metric != SVSB200_L2;
+    bp.work_counter = d_work.ptr;
+    bp.count_ptr = d_counts.ptr + 1;
+    bp.nodes = d_touched.ptr;
+    const int prune_grid = grid_sm * 16;
+
+    // ---- two passes (index.h:436-439): reverse pruning with alpha 1, then with the configured alpha ----
+    for (int pass = 0; pass < 2; ++pass) {
+        const float reverse_alpha = pass == 0 ? 1.0f : alpha;
+        for (size_t b = 0; b < num_batches; ++b) {
+            const size_t start = std::min(n, batchsize * b), stop = std::min(n, batchsize * (b + 1));
+            if (stop == start) continue;
+            const uint32_t B = uint32_t(stop - start);
+            // 1. generate_neighbors: search ...
+            if (dtype == SVSB200_F32)
+                batch_queries_kernel<SVSB200_F32><<<(B + 7) / 8, 256, 0, stream>>>(d_vectors.ptr, row_stride, uint32_t(dim), qstride, uint32_t(start), B, d_qf.ptr, d_qaux.ptr);
+            else
+                batch_queries_kernel<SVSB200_F16><<<(B + 7) / 8, 256, 0, stream>>>(d_vectors.ptr, row_stride, uint32_t(dim), qstride, uint32_t(start), B, d_qf.ptr, d_qaux.ptr);
+            count_launch();
+            CUDA_TRY(cudaMemsetAsync(d_work.ptr, 0, 4, stream));
+            p.nq = B;
+            CUDA_TRY(dtype == SVSB200_F32 ? launch_build_search<SVSB200_F32>(op, p, cfg) : launch_build_search<SVSB200_F16>(op, p, cfg));
+            // ... pool + prune (always with the configured alpha, vamana_build.h:268-272)
+            CUDA_TRY(cudaMemsetAsync(d_work.ptr, 0, 4, stream));
+            bp.reverse = 0;
+            bp.first = uint32_t(start);
+            bp.count = B;
+            bp.limit = R;
+            bp.alpha = alpha;
+            CUDA_TRY(dtype == SVSB200_F32 ? launch_build_prune_op<SVSB200_F32>(op, p, bp, std::min<int>(prune_grid, int(B)), stream)
+                                          : launch_build_prune_op<SVSB200_F16>(op, p, bp, std::min<int>(prune_grid, int(B)), stream));
+            // 2. add_reverse_edges
+            CUDA_TRY(cudaMemsetAsync(d_counts.ptr, 0, 8, stream));
+            reverse_insert_kernel<<<unsigned((size_t(B) * R + 255) / 256), 256, 0, stream>>>(
+                uint32_t(start), B, d_graph.ptr, d_deg.ptr, gstride, R, d_head.ptr, d_next.ptr, d_pair_v.ptr, d_counts.ptr,
+                d_touched.ptr, d_counts.ptr + 1, uint32_t(pair_cap));
+            count_launch();
+            CUDA_TRY(cudaMemsetAsync(d_work.ptr, 0, 4, stream));
+            bp.reverse = 1;
+            bp.limit = uint32_t(prune_to);
+            bp.alpha = reverse_alpha;
+            CUDA_TRY(dtype == SVSB200_F32 ? launch_build_prune_op<SVSB200_F32>(op, p, bp, prune_grid, stream)
+                                          : launch_build_prune_op<SVSB200_F16>(op, p, bp, prune_grid, stream));
+            reset_heads_kernel<<<unsigned((pair_cap + 255) / 256), 256, 0, stream>>>(d_touched.ptr, d_counts.ptr + 1, d_head.ptr);
+            count_launch();
+            CUDA_TRY(cudaGetLastError());
+        }
+    }
+    // ---- export in the reference's layout ----
+    CUDA_TRY(d_export.ensure(n * size_t(R + 1)));
+    export_graph_kernel<<<unsigned((n + 7) / 8), 256, 0, stream>>>(d_graph.ptr, d_deg.ptr, uint32_t(n), gstride, R, d_export.ptr);
+    count_launch();
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaMemcpyAsync(graph_rows_out, d_export.ptr, n * size_t(R + 1) * 4, cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    *entry_point_out = entry_point;
+    return 0;
 }

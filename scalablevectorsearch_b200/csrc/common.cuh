@@ -7,6 +7,7 @@
 #include <cstddef>
 #include <cstdint>
 #include <cstdio>
+#include <memory>
 #include <string>
 
 #include "../../include/svsb200.h"
@@ -44,8 +45,9 @@ struct SearchParams {
     int greater;               // comparator std::greater (IP / cosine): keys are negated
     int sq;                    // rows are scalar-quantised codes
     int lvq;                   // rows are LVQ-8 (mean-removed, per-vector delta/lower)
-    int no_split;              // tuning: keep wide rows on the narrow (G threads per row) mapping
-    float scale, bias, scale_sq;
+    // (scale_sq first: with scale and bias on one 8-byte boundary nvcc pairs their loads, and the search kernels'
+    // register allocation shifts)
+    float scale_sq, scale, bias;
     // prepared queries (output of prepare_queries)
     const float* qf;           // [nq][qstride] fp32 operands of the float tree
     const uint8_t* qcodes;     // [nq][qstride] int8/uint8 operands of the integer kernels
@@ -129,5 +131,78 @@ uint32_t flat_kc();
 
 void count_launch();
 int set_error(const std::string& msg);   // records the calling thread's svsb200_last_error(); returns 1
+
+// A failed CUDA call becomes the calling thread's error, and the enclosing function returns 1.
+#define CUDA_TRY(expr)                                                                         \
+    do {                                                                                       \
+        cudaError_t err__ = (expr);                                                            \
+        if (err__ != cudaSuccess) {                                                            \
+            return set_error(std::string(#expr) + ": " + cudaGetErrorString(err__));           \
+        }                                                                                      \
+    } while (0)
+
+// Owns one device allocation.  The owner selects the allocation's device before the destructor runs.
+template <typename T> struct DeviceBuffer {
+    T* ptr = nullptr;
+    size_t count = 0;
+    DeviceBuffer() = default;
+    DeviceBuffer(const DeviceBuffer&) = delete;
+    DeviceBuffer& operator=(const DeviceBuffer&) = delete;
+    DeviceBuffer(DeviceBuffer&& o) noexcept : ptr(o.ptr), count(o.count) {
+        o.ptr = nullptr;
+        o.count = 0;
+    }
+    ~DeviceBuffer() { release(); }
+    // Room for at least n elements; the old contents are not kept.
+    cudaError_t ensure(size_t n) {
+        if (n <= count) return cudaSuccess;
+        release();   // (cudaFree synchronises the device: safe against work still using the old block)
+        cudaError_t err = cudaMalloc(&ptr, n * sizeof(T));
+        if (err == cudaSuccess) count = n;
+        else ptr = nullptr;
+        return err;
+    }
+    void release() {
+        if (ptr) cudaFree(ptr);
+        ptr = nullptr;
+        count = 0;
+    }
+};
+
+// Owns a stream: StreamOwner owner(stream, cudaStreamDestroy).
+using StreamOwner = std::unique_ptr<CUstream_st, cudaError_t (*)(cudaStream_t)>;
+
+inline size_t esize(int dtype) { return dtype == SVSB200_F32 ? 4 : dtype == SVSB200_F16 ? 2 : 1; }
+inline size_t round_up(size_t x, size_t m) { return (x + m - 1) / m * m; }
+
+// ---- index layout in HBM, shared by the search library and the graph builder ----
+// Bytes from one vector to the next: LVQ-8 rows use the ABI's stride, other rows are padded to 16 bytes.
+inline uint32_t row_stride_for(int storage, int dtype, size_t dim) {
+    return uint32_t(storage == SVSB200_LVQ8 ? svsb200_lvq8_row_stride(dim) : round_up(dim * esize(dtype), 16));
+}
+// Words from one adjacency row to the next.  Rows of up to 128 neighbours are padded to whole 32-word groups (one
+// coalesced load per group and lane in the lean kernel, no per-lane bounds checks); wider rows stay 16-byte aligned.
+inline uint32_t gstride_for(size_t max_degree) {
+    return uint32_t(round_up(max_degree, max_degree <= 32u * kFastMaxGW ? 32 : 4));
+}
+// Elements from one prepared query to the next.
+inline uint32_t qstride_for(size_t dim) { return uint32_t(round_up(dim, 16)); }
+
+// Visited filter of the lean kernel: sets of eight 16-bit tags, `slots` of them (0 = off, else at least 64), doubled
+// until every id >> shift fits below the 0xFFFF "empty" tag, so that the filter is exact.
+struct LeanFilterPlan {
+    uint32_t slots, shift;
+    size_t smem_bytes;   // per CTA
+};
+inline LeanFilterPlan lean_filter_plan(size_t n, size_t dim, size_t capacity, uint32_t deg_pad, uint32_t slots) {
+    if (slots && slots < 64) slots = 64;
+    uint32_t shift = 0;
+    while ((8u << shift) < slots) ++shift;   // log2(sets)
+    while (slots && (uint64_t(n - 1) >> shift) >= 0xFFFFull && shift < 20) {
+        ++shift;
+        slots <<= 1;
+    }
+    return {slots, shift, fast_smem_bytes(qstride_for(dim), uint32_t(round_up(capacity, 32)), deg_pad, slots * 2u)};
+}
 
 }  // namespace svsb200

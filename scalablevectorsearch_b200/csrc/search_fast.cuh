@@ -408,7 +408,7 @@ template <int ROWT, int OP, bool HIST = false> cudaError_t launch_fast_dims(cons
     if constexpr (OP < OP_L2I) {
         if (p.dim == 96) return launch_fast<ROWT, OP, 96, 1, HIST>(p, cfg);
         if (p.dim == 128 && !HIST) return launch_fast<ROWT, OP, 128, 1, HIST>(p, cfg);
-        if (p.dim >= 256 && !p.no_split) return launch_fast<ROWT, OP, 0, 4, HIST>(p, cfg);
+        if (p.dim >= 256) return launch_fast<ROWT, OP, 0, 4, HIST>(p, cfg);
     }
     return launch_fast<ROWT, OP, 0, 1, HIST>(p, cfg);
 }

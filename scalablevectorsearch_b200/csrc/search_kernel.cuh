@@ -933,7 +933,7 @@ template <int ROWT, int OP> cudaError_t launch_dims(const SearchParams& p, const
         if (p.dim == 96) return nrows == 1 ? launch_one<ROWT, OP, 96, 1>(p, cfg) : launch_one<ROWT, OP, 96, 2>(p, cfg);
         if (p.dim == 128) return nrows == 1 ? launch_one<ROWT, OP, 128, 1>(p, cfg) : launch_one<ROWT, OP, 128, 2>(p, cfg);
         // wide rows: accumulators split over 4x the threads (float_rows_split)
-        if (p.dim >= 256 && !p.no_split) return launch_one<ROWT, OP, 0, 2, 4>(p, cfg);
+        if (p.dim >= 256) return launch_one<ROWT, OP, 0, 2, 4>(p, cfg);
     }
     return nrows == 1 ? launch_one<ROWT, OP, 0, 1>(p, cfg) : launch_one<ROWT, OP, 0, 2>(p, cfg);
 }

@@ -23,6 +23,7 @@
 #include <memory>
 #include <mutex>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include <sys/stat.h>
@@ -38,36 +39,6 @@ static int fail(const std::string& msg) {
     return 1;
 }
 int set_error(const std::string& msg) { return fail(msg); }
-#define CUDA_TRY(expr)                                                                         \
-    do {                                                                                       \
-        cudaError_t err__ = (expr);                                                            \
-        if (err__ != cudaSuccess) {                                                            \
-            return fail(std::string(#expr) + ": " + cudaGetErrorString(err__));                \
-        }                                                                                      \
-    } while (0)
-
-static size_t esize(int dtype) { return dtype == SVSB200_F32 ? 4 : dtype == SVSB200_F16 ? 2 : 1; }
-static size_t round_up(size_t x, size_t m) { return (x + m - 1) / m * m; }
-
-template <typename T> struct DeviceBuffer {
-    T* ptr = nullptr;
-    size_t count = 0;
-    cudaError_t ensure(size_t n) {
-        if (n <= count) return cudaSuccess;
-        if (ptr) cudaFree(ptr);   // (synchronises the device: safe against work still using the old block)
-        ptr = nullptr;
-        count = 0;
-        cudaError_t err = cudaMalloc(&ptr, n * sizeof(T));
-        if (err == cudaSuccess) count = n;
-        return err;
-    }
-    void release() {
-        if (ptr) cudaFree(ptr);
-        ptr = nullptr;
-        count = 0;
-    }
-};
-
 // Everything one in-flight search needs on one device: the analogue of the reference's per-thread scratch
 // space (index/vamana/index.h:455-470).
 struct Scratch {
@@ -87,23 +58,15 @@ struct Scratch {
     DeviceBuffer<uint64_t> flat_i2;
     DeviceBuffer<uint64_t> gather_ids, merged_ids;     // sharded search (on the merging device)
     DeviceBuffer<float> gather_dists, merged_dists;
-    unsigned int* d_counter = nullptr;
-    int* d_cancel = nullptr;
+    DeviceBuffer<unsigned int> d_counter;
+    DeviceBuffer<int> d_cancel;
     cudaEvent_t ev_start = nullptr, ev_stop = nullptr, ev_done = nullptr;
     bool timed = false;
     bool poll_cancel = false;        // this search was given a cancellation predicate: the kernels poll the flag
     size_t counted_nq = 0;
     int last_kernel = 0;
-    ~Scratch() {
+    ~Scratch() {   // (the buffers are freed after this body, on the device it selects)
         cudaSetDevice(device);
-        q_raw.release(); q_codes.release(); ids.release(); q_f32.release(); q_aux.release(); dists.release();
-        hops.release(); evals.release(); fetched.release();
-        gather_ids.release(); merged_ids.release(); gather_dists.release(); merged_dists.release();
-        exh_ids.release(); exh_dists.release();
-        flat_a.release(); flat_q2.release(); flat_qnorm.release(); flat_ckey.release(); flat_d2.release();
-        flat_cid.release(); flat_unv.release(); flat_i2.release(); flat_progress.release();
-        if (d_counter) cudaFree(d_counter);
-        if (d_cancel) cudaFree(d_cancel);
         if (ev_start) cudaEventDestroy(ev_start);
         if (ev_stop) cudaEventDestroy(ev_stop);
         if (ev_done) cudaEventDestroy(ev_done);
@@ -116,31 +79,20 @@ struct Scratch {
 struct Replica {
     int device = 0;
     int sm_count = 0;
-    void* d_vectors = nullptr;
-    uint32_t* d_graph = nullptr;
-    uint16_t* d_ref_degree = nullptr;
-    float* d_mean = nullptr;          // LVQ-8: dataset mean
-    uint32_t* d_entry = nullptr;      // entry points when there are several
+    DeviceBuffer<char> d_vectors;
+    DeviceBuffer<uint32_t> d_graph;
+    DeviceBuffer<uint16_t> d_ref_degree;
+    DeviceBuffer<float> d_mean;          // LVQ-8: dataset mean
+    DeviceBuffer<uint32_t> d_entry;      // entry points when there are several
     // tensor-core flat search: the base vectors as fp16 UMMA tiles + per-row bias, built on first use
-    void* flat_b = nullptr;
-    float* flat_bias = nullptr;
-    unsigned int* flat_xmax = nullptr;
+    DeviceBuffer<char> flat_b;
+    DeviceBuffer<float> flat_bias;
+    DeviceBuffer<unsigned int> flat_xmax;
     std::mutex mu;
     std::vector<Scratch*> idle;                      // pool for the blocking API
     std::map<cudaStream_t, Scratch*> by_stream;      // one per caller stream for the enqueue-only API
-    std::vector<std::unique_ptr<Scratch>> all;
-    ~Replica() {
-        cudaSetDevice(device);
-        all.clear();
-        if (d_vectors) cudaFree(d_vectors);
-        if (d_graph) cudaFree(d_graph);
-        if (d_ref_degree) cudaFree(d_ref_degree);
-        if (d_mean) cudaFree(d_mean);
-        if (d_entry) cudaFree(d_entry);
-        if (flat_b) cudaFree(flat_b);
-        if (flat_bias) cudaFree(flat_bias);
-        if (flat_xmax) cudaFree(flat_xmax);
-    }
+    std::vector<std::unique_ptr<Scratch>> all;       // (declared last: destroyed before the arrays above)
+    ~Replica() { cudaSetDevice(device); }
 };
 
 }  // namespace svsb200
@@ -160,7 +112,7 @@ struct svsb200_index {
     std::vector<std::unique_ptr<Replica>> reps;
     int counting = 0;
     // options
-    long warps_per_cta = 0, ctas_per_sm = 0, rows_in_flight = 0, filter_slots = -1, filter_tag16 = 1, no_split = 0;
+    long warps_per_cta = 0, ctas_per_sm = 0, rows_in_flight = 0, filter_slots = -1;
     long generic_kernel = 0;          // 1: force the generic (round-1) kernel instead of the lean one
     long host_chunks = 0;             // host-buffer searches: pieces per device whose copies overlap the kernels (0 = auto)
     std::mutex mu;
@@ -169,7 +121,8 @@ struct svsb200_index {
 
 namespace svsb200 {
 
-static Scratch* new_scratch(Replica* rep, cudaStream_t caller_stream, std::string* err) {
+// A new scratch set of the replica (null, with the error recorded, when it cannot be made).
+static Scratch* new_scratch(Replica* rep, cudaStream_t caller_stream) {
     auto sc = std::make_unique<Scratch>();
     sc->device = rep->device;
     cudaError_t e = cudaSuccess;
@@ -180,14 +133,14 @@ static Scratch* new_scratch(Replica* rep, cudaStream_t caller_stream, std::strin
         sc->owns_stream = true;
     }
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&sc->ctl, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaMalloc(&sc->d_counter, sizeof(unsigned int));
-    if (e == cudaSuccess) e = cudaMalloc(&sc->d_cancel, sizeof(int));
-    if (e == cudaSuccess) e = cudaMemset(sc->d_cancel, 0, sizeof(int));
+    if (e == cudaSuccess) e = sc->d_counter.ensure(1);
+    if (e == cudaSuccess) e = sc->d_cancel.ensure(1);
+    if (e == cudaSuccess) e = cudaMemset(sc->d_cancel.ptr, 0, sizeof(int));
     if (e == cudaSuccess) e = cudaEventCreate(&sc->ev_start);
     if (e == cudaSuccess) e = cudaEventCreate(&sc->ev_stop);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&sc->ev_done, cudaEventDisableTiming);
     if (e != cudaSuccess) {
-        *err = std::string("scratch allocation: ") + cudaGetErrorString(e);
+        fail(std::string("scratch allocation: ") + cudaGetErrorString(e));
         return nullptr;
     }
     Scratch* raw = sc.get();
@@ -195,28 +148,54 @@ static Scratch* new_scratch(Replica* rep, cudaStream_t caller_stream, std::strin
     return raw;
 }
 
-// Blocking API: any idle scratch of the replica (a new one if all are busy -- one per concurrent caller).
-static Scratch* acquire(Replica* rep, std::string* err) {
-    std::lock_guard<std::mutex> lock(rep->mu);
-    if (!rep->idle.empty()) {
-        Scratch* sc = rep->idle.back();
-        rep->idle.pop_back();
-        return sc;
-    }
-    return new_scratch(rep, nullptr, err);
-}
-static void release(Replica* rep, Scratch* sc) {
-    std::lock_guard<std::mutex> lock(rep->mu);
-    rep->idle.push_back(sc);
-}
 // Enqueue-only API: the scratch bound to the caller's stream (work on one stream is ordered, so it is reusable).
-static Scratch* scratch_for_stream(Replica* rep, cudaStream_t stream, std::string* err) {
+static Scratch* scratch_for_stream(Replica* rep, cudaStream_t stream) {
     std::lock_guard<std::mutex> lock(rep->mu);
     auto it = rep->by_stream.find(stream);
     if (it != rep->by_stream.end()) return it->second;
-    Scratch* sc = new_scratch(rep, stream, err);
+    Scratch* sc = new_scratch(rep, stream);
     if (sc) rep->by_stream[stream] = sc;
     return sc;
+}
+
+// The scratch set of one blocking call.  With a caller stream it is the one bound to that stream; without, it is an
+// idle one of the replica's pool (a new one if all are busy -- one per concurrent caller), which goes back to the pool
+// when the lease ends.  take() also selects the replica's device.
+struct ScratchLease {
+    Scratch* sc = nullptr;
+    Replica* pool = nullptr;   // set while `sc` is checked out of this replica's pool
+    ScratchLease() = default;
+    ScratchLease(ScratchLease&& o) noexcept : sc(o.sc), pool(o.pool) { o.pool = nullptr; }
+    ~ScratchLease() {
+        if (!pool) return;
+        std::lock_guard<std::mutex> lock(pool->mu);
+        pool->idle.push_back(sc);
+    }
+    int take(Replica* rep, cudaStream_t caller_stream) {
+        CUDA_TRY(cudaSetDevice(rep->device));
+        if (caller_stream) {
+            sc = scratch_for_stream(rep, caller_stream);
+        } else {
+            std::lock_guard<std::mutex> lock(rep->mu);
+            if (rep->idle.empty()) {
+                sc = new_scratch(rep, nullptr);
+            } else {
+                sc = rep->idle.back();
+                rep->idle.pop_back();
+            }
+            if (sc) pool = rep;
+        }
+        return sc ? 0 : 1;
+    }
+};
+
+// The scratch set of an enqueue-only call: the one bound to the caller's stream (NULL: a stream the index keeps for
+// that purpose) on the index's only device, which is selected.
+static int device_api_scratch(const char* who, svsb200_index* ix, void* stream, Scratch** sc) {
+    if (ix->reps.size() != 1) return fail(std::string(who) + ": the index must live on exactly one device");
+    CUDA_TRY(cudaSetDevice(ix->reps[0]->device));
+    *sc = scratch_for_stream(ix->reps[0].get(), static_cast<cudaStream_t>(stream));
+    return *sc ? 0 : 1;
 }
 
 // threads::balance (lib/threads/types.h:311-329): contiguous ranges whose sizes differ by at most one.
@@ -470,6 +449,15 @@ __global__ void merge_topk_kernel(const uint64_t* __restrict__ ids, const float*
     }
 }
 
+static cudaError_t launch_merge_topk(const uint64_t* ids, const float* dists, size_t nshards, size_t nq, size_t k, int greater,
+                                     uint64_t* out_ids, float* out_dists, cudaStream_t stream) {
+    const unsigned warps = 4;
+    merge_topk_kernel<<<unsigned((nq + warps - 1) / warps), warps * 32, 0, stream>>>(
+        ids, dists, uint32_t(nshards), uint32_t(nq), uint32_t(k), greater, out_ids, out_dists);
+    count_launch();
+    return cudaGetLastError();
+}
+
 // LVQ-8 encoder (own specification, DESIGN.md §10), one warp per vector:
 //   r_i = x_i - mean_i;  lower = min r, upper = max r;  delta = (upper - lower) / 255
 //   {delta, lower} are stored as float16 (round to nearest even) and the codes are computed against
@@ -563,16 +551,39 @@ __global__ void range_count_kernel(const float* __restrict__ dists, const uint64
     if (c == kk && !exhausted) atomicAdd(unfinished, 1u);
 }
 
-template <int QT>
-static cudaError_t launch_prepare(const void* d_queries, uint32_t nq, uint32_t dim, uint32_t qstride, int mode, int metric,
-                                  int code_type, float scale, float bias, const float* mean, float* qf, uint8_t* qcodes,
-                                  float* qaux, cudaStream_t stream) {
-    const int warps = 8;
-    const unsigned grid = (nq + warps - 1) / warps;
-    prepare_queries_kernel<QT><<<grid, warps * 32, 0, stream>>>(d_queries, nq, dim, qstride, mode, metric, code_type, scale,
-                                                               bias, mean, qf, qcodes, qaux);
+// Prepares the batch's queries for the search kernels (the device-side maybe_fix_argument) into sc's query buffers.
+static int prepare_queries(const svsb200_index* ix, const Replica* rep, Scratch* sc, const void* d_queries, int qdtype,
+                           size_t nq, int mode, cudaStream_t stream) {
+    const uint32_t qstride = qstride_for(ix->dim);
+    CUDA_TRY(sc->q_f32.ensure(nq * qstride));
+    CUDA_TRY(sc->q_codes.ensure(nq * qstride));
+    CUDA_TRY(sc->q_aux.ensure(nq * 2));
+    auto launch = [&](auto kernel) {
+        const int warps = 8;
+        kernel<<<unsigned((nq + warps - 1) / warps), warps * 32, 0, stream>>>(
+            d_queries, uint32_t(nq), uint32_t(ix->dim), qstride, mode, ix->metric, ix->dtype, ix->scale, ix->bias,
+            rep->d_mean.ptr, sc->q_f32.ptr, sc->q_codes.ptr, sc->q_aux.ptr);
+    };
+    switch (qdtype) {
+        case SVSB200_F32: launch(prepare_queries_kernel<SVSB200_F32>); break;
+        case SVSB200_F16: launch(prepare_queries_kernel<SVSB200_F16>); break;
+        case SVSB200_I8: launch(prepare_queries_kernel<SVSB200_I8>); break;
+        default: launch(prepare_queries_kernel<SVSB200_U8>);
+    }
     count_launch();
-    return cudaGetLastError();
+    CUDA_TRY(cudaGetLastError());
+    return 0;
+}
+
+// Calls f(std::integral_constant<int, ROWT>()) for the search kernels' row type `rowt`.
+template <typename F> static cudaError_t with_row_type(int rowt, F&& f) {
+    switch (rowt) {
+        case ROW_LVQ8: return f(std::integral_constant<int, ROW_LVQ8>());
+        case SVSB200_F32: return f(std::integral_constant<int, SVSB200_F32>());
+        case SVSB200_F16: return f(std::integral_constant<int, SVSB200_F16>());
+        case SVSB200_I8: return f(std::integral_constant<int, SVSB200_I8>());
+        default: return f(std::integral_constant<int, SVSB200_U8>());
+    }
 }
 
 }  // namespace svsb200
@@ -600,149 +611,6 @@ int svsb200_device_sm(int device, int* sm) {
     CUDA_TRY(cudaGetDeviceProperties(&prop, device));
     if (sm) *sm = prop.major * 10 + prop.minor;
     return 0;
-}
-
-// Uploads one replica from the host arrays.
-static int upload_replica(svsb200_index* ix, Replica* rep, const void* vectors, size_t src_stride, size_t row_bytes,
-                          const uint32_t* graph_rows, size_t graph_row_len, const float* aux) {
-    const size_t n = ix->n;
-    CUDA_TRY(cudaSetDevice(rep->device));
-    const size_t vbytes = n * size_t(ix->row_stride);
-    const size_t gbytes = n * size_t(ix->gstride) * sizeof(uint32_t);
-    CUDA_TRY(cudaMalloc(&rep->d_vectors, vbytes));
-    CUDA_TRY(cudaMalloc(&rep->d_graph, gbytes));
-    CUDA_TRY(cudaMalloc(&rep->d_ref_degree, n * sizeof(uint16_t)));
-    ix->device_bytes = vbytes + gbytes + n * sizeof(uint16_t);
-    CUDA_TRY(cudaMemset(rep->d_vectors, 0, vbytes));
-    CUDA_TRY(cudaMemcpy2D(rep->d_vectors, ix->row_stride, vectors, src_stride, row_bytes, n, cudaMemcpyHostToDevice));
-    {
-        uint32_t* d_src = nullptr;
-        int* d_bad = nullptr;
-        const size_t sbytes = n * graph_row_len * sizeof(uint32_t);
-        CUDA_TRY(cudaMalloc(&d_src, sbytes));
-        cudaError_t err = cudaMalloc(&d_bad, sizeof(int));
-        if (err == cudaSuccess) err = cudaMemset(d_bad, 0, sizeof(int));
-        if (err == cudaSuccess) err = cudaMemcpy(d_src, graph_rows, sbytes, cudaMemcpyHostToDevice);
-        int bad = 0;
-        if (err == cudaSuccess) {
-            const int warps = 8;
-            repack_graph_kernel<<<unsigned((n + warps - 1) / warps), warps * 32>>>(d_src, graph_row_len, uint32_t(n),
-                                                                                  rep->d_graph, ix->gstride,
-                                                                                  rep->d_ref_degree, d_bad);
-            count_launch();
-            err = cudaGetLastError();
-        }
-        if (err == cudaSuccess) err = cudaMemcpy(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost);
-        cudaFree(d_src);
-        if (d_bad) cudaFree(d_bad);
-        CUDA_TRY(err);
-        if (bad)
-            return fail(bad == 1 ? "svsb200_index_create: adjacency row with degree > max_degree"
-                                 : "svsb200_index_create: neighbour id out of range");
-    }
-    if (ix->storage == SVSB200_LVQ8) {
-        CUDA_TRY(cudaMalloc(&rep->d_mean, ix->dim * sizeof(float)));
-        CUDA_TRY(cudaMemcpy(rep->d_mean, aux, ix->dim * sizeof(float), cudaMemcpyHostToDevice));
-    }
-    return 0;
-}
-
-// Copies an uploaded replica device to device (NVLink when peer access exists).
-static int clone_replica(svsb200_index* ix, const Replica* src, Replica* dst) {
-    const size_t n = ix->n;
-    CUDA_TRY(cudaSetDevice(dst->device));
-    const size_t vbytes = n * size_t(ix->row_stride);
-    const size_t gbytes = n * size_t(ix->gstride) * sizeof(uint32_t);
-    CUDA_TRY(cudaMalloc(&dst->d_vectors, vbytes));
-    CUDA_TRY(cudaMalloc(&dst->d_graph, gbytes));
-    CUDA_TRY(cudaMalloc(&dst->d_ref_degree, n * sizeof(uint16_t)));
-    CUDA_TRY(cudaMemcpyPeer(dst->d_vectors, dst->device, src->d_vectors, src->device, vbytes));
-    CUDA_TRY(cudaMemcpyPeer(dst->d_graph, dst->device, src->d_graph, src->device, gbytes));
-    CUDA_TRY(cudaMemcpyPeer(dst->d_ref_degree, dst->device, src->d_ref_degree, src->device, n * sizeof(uint16_t)));
-    if (src->d_mean) {
-        CUDA_TRY(cudaMalloc(&dst->d_mean, ix->dim * sizeof(float)));
-        CUDA_TRY(cudaMemcpyPeer(dst->d_mean, dst->device, src->d_mean, src->device, ix->dim * sizeof(float)));
-    }
-    return 0;
-}
-
-int svsb200_index_create_multi(const void* vectors, int dtype, size_t n, size_t dim, size_t row_stride_bytes,
-                               const uint32_t* graph_rows, size_t graph_row_len, uint32_t entry_point, int metric,
-                               int storage, const float* aux, const int* devices, size_t ndevices, svsb200_index** out) {
-    if (!out) return fail("svsb200_index_create: out is NULL");
-    *out = nullptr;
-    if (!vectors || !graph_rows) return fail("svsb200_index_create: NULL input");
-    if (!devices || ndevices == 0) return fail("svsb200_index_create: empty device list");
-    if (dtype < SVSB200_F32 || dtype > SVSB200_U8) return fail("svsb200_index_create: bad dtype");
-    if (metric < SVSB200_L2 || metric > SVSB200_COSINE) return fail("svsb200_index_create: bad metric");
-    if (n == 0 || dim == 0) return fail("svsb200_index_create: empty dataset");
-    if (n >= (size_t(1) << 31)) return fail("svsb200_index_create: more than 2^31-1 vectors per index");
-    if (graph_row_len < 2) return fail("svsb200_index_create: graph rows need a degree word and one slot");
-    if (graph_row_len > 65536) return fail("svsb200_index_create: max_degree above 65535");
-    if (entry_point >= n) return fail("svsb200_index_create: entry point out of range");
-    if (storage == SVSB200_SQ) {
-        if (dtype != SVSB200_I8 && dtype != SVSB200_U8) return fail("svsb200_index_create: SQ codes must be int8/uint8");
-        if (!aux) return fail("svsb200_index_create: SQ needs aux = {scale, bias}");
-    } else if (storage == SVSB200_LVQ8) {
-        if (dtype != SVSB200_U8) return fail("svsb200_index_create: LVQ-8 rows are uint8 codes (dtype SVSB200_U8)");
-        if (!aux) return fail("svsb200_index_create: LVQ-8 needs aux = mean[dim]");
-        if (row_stride_bytes != svsb200_lvq8_row_stride(dim))
-            return fail("svsb200_index_create: LVQ-8 rows must use svsb200_lvq8_row_stride(dim)");
-    } else if (storage != SVSB200_PLAIN) {
-        return fail("svsb200_index_create: unsupported storage kind");
-    }
-    const int ndev = svsb200_device_count();
-    if (ndev == 0) return fail("svsb200_index_create: no CUDA device (there is no CPU fallback)");
-
-    std::unique_ptr<svsb200_index> ix(new svsb200_index());
-    ix->dtype = dtype;
-    ix->metric = metric;
-    ix->storage = storage;
-    ix->n = n;
-    ix->dim = dim;
-    ix->max_degree = graph_row_len - 1;
-    ix->entry_point = entry_point;
-    if (storage == SVSB200_SQ) {
-        ix->scale = aux[0];
-        ix->bias = aux[1];
-    }
-    size_t row_bytes = dim * esize(dtype);
-    if (storage == SVSB200_LVQ8) {
-        ix->lvq_const_offset = uint32_t(round_up(dim, 4));
-        row_bytes = ix->lvq_const_offset + 4;
-    }
-    const size_t src_stride = row_stride_bytes ? row_stride_bytes : row_bytes;
-    ix->row_stride = uint32_t(storage == SVSB200_LVQ8 ? svsb200_lvq8_row_stride(dim) : round_up(row_bytes, 16));
-    // rows of up to 128 neighbours are padded to whole 32-word groups (one coalesced load per group and lane in
-    // the lean kernel, no per-lane bounds checks); wider rows stay 16-byte aligned only
-    ix->gstride = uint32_t(round_up(ix->max_degree, ix->max_degree <= 32u * kFastMaxGW ? 32 : 4));
-
-    for (size_t r = 0; r < ndevices; ++r) {
-        const int device = devices[r];
-        if (device < 0 || device >= ndev) return fail("svsb200_index_create: bad device ordinal");
-        for (size_t j = 0; j < r; ++j)
-            if (devices[j] == device) return fail("svsb200_index_create: device listed twice");
-        cudaDeviceProp prop;
-        CUDA_TRY(cudaGetDeviceProperties(&prop, device));
-        if (prop.major != 10 || prop.minor != 0)
-            return fail("svsb200_index_create: device is not sm_100 (this binary holds sm_100a code only)");
-        std::unique_ptr<Replica> rep(new Replica());
-        rep->device = device;
-        rep->sm_count = prop.multiProcessorCount;
-        int rc = r == 0 ? upload_replica(ix.get(), rep.get(), vectors, src_stride, row_bytes, graph_rows, graph_row_len, aux)
-                        : clone_replica(ix.get(), ix->reps[0].get(), rep.get());
-        if (rc) return rc;
-        ix->reps.push_back(std::move(rep));
-    }
-    *out = ix.release();
-    return 0;
-}
-
-int svsb200_index_create(const void* vectors, int dtype, size_t n, size_t dim, size_t row_stride_bytes,
-                         const uint32_t* graph_rows, size_t graph_row_len, uint32_t entry_point, int metric, int storage,
-                         const float* aux, int device, svsb200_index** out) {
-    return svsb200_index_create_multi(vectors, dtype, n, dim, row_stride_bytes, graph_rows, graph_row_len, entry_point,
-                                      metric, storage, aux, &device, 1, out);
 }
 
 // -----------------------------------------------------------------------------------------------------------------
@@ -821,6 +689,20 @@ bool parse_toml_subset(const std::string& text, std::map<std::string, std::strin
         out[table.empty() ? key : table + "." + key] = value;
     }
     return true;
+}
+
+// Reads `path` and parses it with parse_toml_subset.
+int read_toml_file(const std::string& path, std::map<std::string, std::string>& cfg) {
+    FILE* f = fopen(path.c_str(), "rb");
+    if (!f) return fail("cannot open " + path);
+    std::string text;
+    char buf[4096];
+    size_t got;
+    while ((got = fread(buf, 1, sizeof(buf), f)) > 0) text.append(buf, got);
+    fclose(f);
+    std::string err;
+    if (!parse_toml_subset(text, cfg, err)) return fail(path + ": " + err);
+    return 0;
 }
 
 struct RowFile {
@@ -906,18 +788,191 @@ int stream_rows_to_device(RowFile& rf, char* dst, size_t dst_stride, cudaStream_
 
 }  // namespace
 
+// Where the first replica's bytes come from: host arrays, or (when the RowFile pointers are set) the files being
+// assembled from.
+struct ReplicaSource {
+    const void* vectors = nullptr;
+    size_t vector_stride = 0;            // bytes between host rows; 0 = packed
+    const uint32_t* graph_rows = nullptr;
+    const float* aux = nullptr;          // SQ: {scale, bias}; LVQ-8: mean[dim]
+    RowFile* vector_file = nullptr;
+    RowFile* graph_file = nullptr;
+};
+
+// Allocates the replica's arrays and fills them from `src`: the vectors into padded rows, the graph through a staging
+// copy of the reference's rows that repack_graph_kernel turns into the HBM layout.
+static int upload_replica(const char* who, svsb200_index* ix, Replica* rep, size_t graph_row_len, const ReplicaSource& src) {
+    const size_t n = ix->n;
+    CUDA_TRY(cudaSetDevice(rep->device));
+    cudaStream_t stream = nullptr;
+    CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+    StreamOwner stream_owner(stream, cudaStreamDestroy);   // (declared first: destroyed after the staging buffers are freed)
+    const size_t vbytes = n * size_t(ix->row_stride);
+    const size_t gbytes = n * size_t(ix->gstride) * sizeof(uint32_t);
+    CUDA_TRY(rep->d_vectors.ensure(vbytes));
+    CUDA_TRY(rep->d_graph.ensure(n * size_t(ix->gstride)));
+    CUDA_TRY(rep->d_ref_degree.ensure(n));
+    ix->device_bytes = vbytes + gbytes + n * sizeof(uint16_t);
+    CUDA_TRY(cudaMemsetAsync(rep->d_vectors.ptr, 0, vbytes, stream));
+    if (src.vector_file) {
+        if (int rc = stream_rows_to_device(*src.vector_file, rep->d_vectors.ptr, ix->row_stride, stream)) return rc;
+    } else {
+        const size_t row_bytes = ix->storage == SVSB200_LVQ8 ? ix->lvq_const_offset + 4 : ix->dim * esize(ix->dtype);
+        CUDA_TRY(cudaMemcpy2DAsync(rep->d_vectors.ptr, ix->row_stride, src.vectors,
+                                   src.vector_stride ? src.vector_stride : row_bytes, row_bytes, n, cudaMemcpyHostToDevice,
+                                   stream));
+    }
+    DeviceBuffer<uint32_t> d_src;
+    DeviceBuffer<int> d_bad;
+    CUDA_TRY(d_src.ensure(n * graph_row_len));
+    CUDA_TRY(d_bad.ensure(1));
+    CUDA_TRY(cudaMemsetAsync(d_bad.ptr, 0, sizeof(int), stream));
+    if (src.graph_file) {
+        if (int rc = stream_rows_to_device(*src.graph_file, reinterpret_cast<char*>(d_src.ptr), graph_row_len * 4, stream))
+            return rc;
+    } else {
+        CUDA_TRY(cudaMemcpyAsync(d_src.ptr, src.graph_rows, n * graph_row_len * sizeof(uint32_t), cudaMemcpyHostToDevice,
+                                 stream));
+    }
+    const int warps = 8;
+    repack_graph_kernel<<<unsigned((n + warps - 1) / warps), warps * 32, 0, stream>>>(
+        d_src.ptr, graph_row_len, uint32_t(n), rep->d_graph.ptr, ix->gstride, rep->d_ref_degree.ptr, d_bad.ptr);
+    count_launch();
+    CUDA_TRY(cudaGetLastError());
+    int bad = 0;
+    CUDA_TRY(cudaMemcpyAsync(&bad, d_bad.ptr, sizeof(int), cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    if (bad) return fail(std::string(who) + (bad == 1 ? ": adjacency row with degree > max_degree" : ": neighbour id out of range"));
+    if (ix->storage == SVSB200_LVQ8) {
+        CUDA_TRY(rep->d_mean.ensure(ix->dim));
+        CUDA_TRY(cudaMemcpy(rep->d_mean.ptr, src.aux, ix->dim * sizeof(float), cudaMemcpyHostToDevice));
+    }
+    return 0;
+}
+
+// Copies an uploaded replica device to device (NVLink when peer access exists).
+static int clone_replica(svsb200_index* ix, const Replica* src, Replica* dst) {
+    const size_t n = ix->n;
+    CUDA_TRY(cudaSetDevice(dst->device));
+    const size_t vbytes = n * size_t(ix->row_stride);
+    const size_t gbytes = n * size_t(ix->gstride) * sizeof(uint32_t);
+    CUDA_TRY(dst->d_vectors.ensure(vbytes));
+    CUDA_TRY(dst->d_graph.ensure(n * size_t(ix->gstride)));
+    CUDA_TRY(dst->d_ref_degree.ensure(n));
+    CUDA_TRY(cudaMemcpyPeer(dst->d_vectors.ptr, dst->device, src->d_vectors.ptr, src->device, vbytes));
+    CUDA_TRY(cudaMemcpyPeer(dst->d_graph.ptr, dst->device, src->d_graph.ptr, src->device, gbytes));
+    CUDA_TRY(cudaMemcpyPeer(dst->d_ref_degree.ptr, dst->device, src->d_ref_degree.ptr, src->device, n * sizeof(uint16_t)));
+    if (src->d_mean.ptr) {
+        CUDA_TRY(dst->d_mean.ensure(ix->dim));
+        CUDA_TRY(cudaMemcpyPeer(dst->d_mean.ptr, dst->device, src->d_mean.ptr, src->device, ix->dim * sizeof(float)));
+    }
+    return 0;
+}
+
+// Argument checks that create and assemble share, in the order both make them.
+static int check_index_kind(const char* who, const int* devices, size_t ndevices, int dtype, int metric) {
+    const std::string w(who);
+    if (!devices || ndevices == 0) return fail(w + ": empty device list");
+    if (dtype < SVSB200_F32 || dtype > SVSB200_U8) return fail(w + ": bad dtype");
+    if (metric < SVSB200_L2 || metric > SVSB200_COSINE) return fail(w + ": bad metric");
+    return 0;
+}
+static int check_index_size(const char* who, size_t n, size_t dim) {
+    if (n == 0 || dim == 0) return fail(std::string(who) + ": empty dataset");
+    if (n >= (size_t(1) << 31)) return fail(std::string(who) + ": more than 2^31-1 vectors per index");
+    return 0;
+}
+
+// The index over checked arguments: its fields and layout, then one replica per listed device, the first uploaded from
+// `src` and the others copied from it.
+static int make_index(const char* who, int dtype, int metric, int storage, size_t n, size_t dim, size_t graph_row_len,
+                      uint32_t entry_point, const int* devices, size_t ndevices, const ReplicaSource& src,
+                      std::unique_ptr<svsb200_index>& ix) {
+    const std::string w(who);
+    const int ndev = svsb200_device_count();
+    if (ndev == 0) return fail(w + ": no CUDA device (there is no CPU fallback)");
+    ix.reset(new svsb200_index());
+    ix->dtype = dtype;
+    ix->metric = metric;
+    ix->storage = storage;
+    ix->n = n;
+    ix->dim = dim;
+    ix->max_degree = graph_row_len - 1;
+    ix->entry_point = entry_point;
+    if (storage == SVSB200_SQ) {
+        ix->scale = src.aux[0];
+        ix->bias = src.aux[1];
+    }
+    if (storage == SVSB200_LVQ8) ix->lvq_const_offset = uint32_t(round_up(dim, 4));
+    ix->row_stride = row_stride_for(storage, dtype, dim);
+    ix->gstride = gstride_for(ix->max_degree);
+
+    for (size_t r = 0; r < ndevices; ++r) {
+        const int device = devices[r];
+        if (device < 0 || device >= ndev) return fail(w + ": bad device ordinal");
+        for (size_t j = 0; j < r; ++j)
+            if (devices[j] == device) return fail(w + ": device listed twice");
+        cudaDeviceProp prop;
+        CUDA_TRY(cudaGetDeviceProperties(&prop, device));
+        if (prop.major != 10 || prop.minor != 0) return fail(w + ": device is not sm_100 (this binary holds sm_100a code only)");
+        std::unique_ptr<Replica> rep(new Replica());
+        rep->device = device;
+        rep->sm_count = prop.multiProcessorCount;
+        int rc = r == 0 ? upload_replica(who, ix.get(), rep.get(), graph_row_len, src)
+                        : clone_replica(ix.get(), ix->reps[0].get(), rep.get());
+        if (rc) return rc;
+        ix->reps.push_back(std::move(rep));
+    }
+    return 0;
+}
+
+int svsb200_index_create_multi(const void* vectors, int dtype, size_t n, size_t dim, size_t row_stride_bytes,
+                               const uint32_t* graph_rows, size_t graph_row_len, uint32_t entry_point, int metric,
+                               int storage, const float* aux, const int* devices, size_t ndevices, svsb200_index** out) {
+    const char* who = "svsb200_index_create";
+    if (!out) return fail("svsb200_index_create: out is NULL");
+    *out = nullptr;
+    if (!vectors || !graph_rows) return fail("svsb200_index_create: NULL input");
+    if (int rc = check_index_kind(who, devices, ndevices, dtype, metric)) return rc;
+    if (int rc = check_index_size(who, n, dim)) return rc;
+    if (graph_row_len < 2) return fail("svsb200_index_create: graph rows need a degree word and one slot");
+    if (graph_row_len > 65536) return fail("svsb200_index_create: max_degree above 65535");
+    if (entry_point >= n) return fail("svsb200_index_create: entry point out of range");
+    if (storage == SVSB200_SQ) {
+        if (dtype != SVSB200_I8 && dtype != SVSB200_U8) return fail("svsb200_index_create: SQ codes must be int8/uint8");
+        if (!aux) return fail("svsb200_index_create: SQ needs aux = {scale, bias}");
+    } else if (storage == SVSB200_LVQ8) {
+        if (dtype != SVSB200_U8) return fail("svsb200_index_create: LVQ-8 rows are uint8 codes (dtype SVSB200_U8)");
+        if (!aux) return fail("svsb200_index_create: LVQ-8 needs aux = mean[dim]");
+        if (row_stride_bytes != svsb200_lvq8_row_stride(dim))
+            return fail("svsb200_index_create: LVQ-8 rows must use svsb200_lvq8_row_stride(dim)");
+    } else if (storage != SVSB200_PLAIN) {
+        return fail("svsb200_index_create: unsupported storage kind");
+    }
+    ReplicaSource src;
+    src.vectors = vectors;
+    src.vector_stride = row_stride_bytes;
+    src.graph_rows = graph_rows;
+    src.aux = aux;
+    std::unique_ptr<svsb200_index> ix;
+    if (int rc = make_index(who, dtype, metric, storage, n, dim, graph_row_len, entry_point, devices, ndevices, src, ix))
+        return rc;
+    *out = ix.release();
+    return 0;
+}
+
+int svsb200_index_create(const void* vectors, int dtype, size_t n, size_t dim, size_t row_stride_bytes,
+                         const uint32_t* graph_rows, size_t graph_row_len, uint32_t entry_point, int metric, int storage,
+                         const float* aux, int device, svsb200_index** out) {
+    return svsb200_index_create_multi(vectors, dtype, n, dim, row_stride_bytes, graph_rows, graph_row_len, entry_point,
+                                      metric, storage, aux, &device, 1, out);
+}
+
+
 int svsb200_toml_get(const char* path, const char* dotted_key, char* out, size_t capacity) {
     if (!path || !dotted_key || !out || capacity == 0) return fail("svsb200_toml_get: NULL argument");
-    FILE* f = fopen(path, "rb");
-    if (!f) return fail(std::string("cannot open ") + path);
-    std::string text;
-    char buf[4096];
-    size_t got;
-    while ((got = fread(buf, 1, sizeof(buf), f)) > 0) text.append(buf, got);
-    fclose(f);
     std::map<std::string, std::string> cfg;
-    std::string err;
-    if (!parse_toml_subset(text, cfg, err)) return fail(std::string(path) + ": " + err);
+    if (int rc = read_toml_file(path, cfg)) return rc;
     auto it = cfg.find(dotted_key);
     if (it == cfg.end()) return fail(std::string(path) + ": no key " + dotted_key);
     if (it->second.size() + 1 > capacity) return fail("svsb200_toml_get: value does not fit");
@@ -927,26 +982,15 @@ int svsb200_toml_get(const char* path, const char* dotted_key, char* out, size_t
 
 int svsb200_index_assemble(const char* config_path, const char* graph_path, const char* data_path, int dtype,
                            size_t expected_dims, int metric, const int* devices, size_t ndevices, svsb200_index** out) {
+    const char* who = "svsb200_index_assemble";
     if (!out) return fail("svsb200_index_assemble: out is NULL");
     *out = nullptr;
     if (!config_path || !graph_path || !data_path) return fail("svsb200_index_assemble: NULL path");
-    if (!devices || ndevices == 0) return fail("svsb200_index_assemble: empty device list");
-    if (dtype < SVSB200_F32 || dtype > SVSB200_U8) return fail("svsb200_index_assemble: bad dtype");
-    if (metric < SVSB200_L2 || metric > SVSB200_COSINE) return fail("svsb200_index_assemble: bad metric");
+    if (int rc = check_index_kind(who, devices, ndevices, dtype, metric)) return rc;
     // ---- VamanaIndexParameters from TOML ----
     const std::string cfg_file = resolve(config_path, "svs_config.toml");
     std::map<std::string, std::string> cfg;
-    {
-        FILE* f = fopen(cfg_file.c_str(), "rb");
-        if (!f) return fail("cannot open " + cfg_file);
-        std::string text;
-        char buf[4096];
-        size_t got;
-        while ((got = fread(buf, 1, sizeof(buf), f)) > 0) text.append(buf, got);
-        fclose(f);
-        std::string err;
-        if (!parse_toml_subset(text, cfg, err)) return fail(cfg_file + ": " + err);
-    }
+    if (int rc = read_toml_file(cfg_file, cfg)) return rc;
     auto cfg_long = [&](const char* key, long dflt) {
         auto it = cfg.find(key);
         if (it == cfg.end()) return dflt;
@@ -966,84 +1010,20 @@ int svsb200_index_assemble(const char* config_path, const char* graph_path, cons
         return fail("svsb200_index_assemble: the data file holds " + std::to_string(data.dim) + "-dimensional vectors, " +
                     std::to_string(expected_dims) + " expected");
     if (graph.n != data.n) return fail("Wrong sizes!");   // index/vamana/index.h:417-419
-    const size_t n = data.n, dim = data.dim, graph_row_len = graph.dim;
-    if (n == 0 || dim == 0) return fail("svsb200_index_assemble: empty dataset");
-    if (n >= (size_t(1) << 31)) return fail("svsb200_index_assemble: more than 2^31-1 vectors per index");
+    const size_t n = data.n, graph_row_len = graph.dim;
+    if ((rc = check_index_size(who, n, data.dim))) return rc;
     if (graph_row_len < 2 || graph_row_len > 65536) return fail("svsb200_index_assemble: bad graph row length");
     if (entry_point < 0 || size_t(entry_point) >= n) return fail("svsb200_index_assemble: entry point out of range");
-    const int ndev = svsb200_device_count();
-    if (ndev == 0) return fail("svsb200_index_assemble: no CUDA device (there is no CPU fallback)");
-
-    std::unique_ptr<svsb200_index> ix(new svsb200_index());
-    ix->dtype = dtype;
-    ix->metric = metric;
-    ix->storage = SVSB200_PLAIN;
-    ix->n = n;
-    ix->dim = dim;
-    ix->max_degree = graph_row_len - 1;
-    ix->entry_point = uint32_t(entry_point);
-    ix->row_stride = uint32_t(round_up(dim * esize(dtype), 16));
-    ix->gstride = uint32_t(round_up(ix->max_degree, ix->max_degree <= 32u * kFastMaxGW ? 32 : 4));
+    ReplicaSource src;
+    src.vector_file = &data;
+    src.graph_file = &graph;
+    std::unique_ptr<svsb200_index> ix;
+    rc = make_index(who, dtype, metric, SVSB200_PLAIN, n, data.dim, graph_row_len, uint32_t(entry_point), devices, ndevices,
+                    src, ix);
+    if (rc) return rc;
     ix->cfg_window = cfg_long("object.search_parameters.search_window_size", 0);
     ix->cfg_capacity = cfg_long("object.search_parameters.search_buffer_capacity", 0);
     ix->cfg_visited = cfg_long("object.search_parameters.search_buffer_visited_set", 0);
-
-    for (size_t r = 0; r < ndevices; ++r) {
-        const int device = devices[r];
-        if (device < 0 || device >= ndev) return fail("svsb200_index_assemble: bad device ordinal");
-        cudaDeviceProp prop;
-        CUDA_TRY(cudaGetDeviceProperties(&prop, device));
-        if (prop.major != 10 || prop.minor != 0)
-            return fail("svsb200_index_assemble: device is not sm_100 (this binary holds sm_100a code only)");
-        std::unique_ptr<Replica> rep(new Replica());
-        rep->device = device;
-        rep->sm_count = prop.multiProcessorCount;
-        if (r > 0) {
-            rc = clone_replica(ix.get(), ix->reps[0].get(), rep.get());
-            if (rc) return rc;
-            ix->reps.push_back(std::move(rep));
-            continue;
-        }
-        CUDA_TRY(cudaSetDevice(device));
-        cudaStream_t stream;
-        CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-        const size_t vbytes = n * size_t(ix->row_stride), gbytes = n * size_t(ix->gstride) * 4;
-        uint32_t* d_src = nullptr;
-        int* d_bad = nullptr;
-        auto body = [&]() -> int {
-            CUDA_TRY(cudaMalloc(&rep->d_vectors, vbytes));
-            CUDA_TRY(cudaMalloc(&rep->d_graph, gbytes));
-            CUDA_TRY(cudaMalloc(&rep->d_ref_degree, n * 2));
-            ix->device_bytes = vbytes + gbytes + n * 2;
-            CUDA_TRY(cudaMemsetAsync(rep->d_vectors, 0, vbytes, stream));
-            int rc2 = stream_rows_to_device(data, static_cast<char*>(rep->d_vectors), ix->row_stride, stream);
-            if (rc2) return rc2;
-            // the graph: streamed into a device staging area, then repacked (degree word dropped, rows padded)
-            CUDA_TRY(cudaMalloc(&d_src, n * graph_row_len * 4));
-            CUDA_TRY(cudaMalloc(&d_bad, 4));
-            CUDA_TRY(cudaMemsetAsync(d_bad, 0, 4, stream));
-            rc2 = stream_rows_to_device(graph, reinterpret_cast<char*>(d_src), graph_row_len * 4, stream);
-            if (rc2) return rc2;
-            const int warps = 8;
-            repack_graph_kernel<<<unsigned((n + warps - 1) / warps), warps * 32, 0, stream>>>(
-                d_src, graph_row_len, uint32_t(n), rep->d_graph, ix->gstride, rep->d_ref_degree, d_bad);
-            count_launch();
-            CUDA_TRY(cudaGetLastError());
-            int bad = 0;
-            CUDA_TRY(cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, stream));
-            CUDA_TRY(cudaStreamSynchronize(stream));
-            if (bad)
-                return fail(bad == 1 ? "svsb200_index_assemble: adjacency row with degree > max_degree"
-                                     : "svsb200_index_assemble: neighbour id out of range");
-            return 0;
-        };
-        rc = body();
-        if (d_src) cudaFree(d_src);
-        if (d_bad) cudaFree(d_bad);
-        cudaStreamDestroy(stream);
-        if (rc) return rc;
-        ix->reps.push_back(std::move(rep));
-    }
     *out = ix.release();
     return 0;
 }
@@ -1074,8 +1054,8 @@ int svsb200_set_entry_points(svsb200_index* ix, const uint32_t* entry_points, si
     for (auto& rep : ix->reps) {
         CUDA_TRY(cudaSetDevice(rep->device));
         CUDA_TRY(cudaDeviceSynchronize());
-        if (!rep->d_entry) CUDA_TRY(cudaMalloc(&rep->d_entry, 32 * sizeof(uint32_t)));
-        CUDA_TRY(cudaMemcpy(rep->d_entry, entry_points, count * sizeof(uint32_t), cudaMemcpyHostToDevice));
+        CUDA_TRY(rep->d_entry.ensure(32));
+        CUDA_TRY(cudaMemcpy(rep->d_entry.ptr, entry_points, count * sizeof(uint32_t), cudaMemcpyHostToDevice));
     }
     ix->entry_point = entry_points[0];
     ix->n_entry = uint32_t(count);
@@ -1100,10 +1080,6 @@ int svsb200_set_option(svsb200_index* ix, const char* name, long value) {
     } else if (key == "rows_in_flight") {
         if (value < 0 || value > 2) return fail("rows_in_flight must be in [0, 2]");
         ix->rows_in_flight = value;
-    } else if (key == "no_split") {
-        ix->no_split = value;
-    } else if (key == "filter_tag16") {
-        ix->filter_tag16 = value;
     } else if (key == "generic_kernel") {
         ix->generic_kernel = value;
     } else if (key == "host_chunks") {
@@ -1188,10 +1164,6 @@ static int search_on_device(svsb200_index* ix, Replica* rep, Scratch* sc, const 
         mode = PREP_FLOAT;
     }
 
-    const uint32_t qstride = uint32_t(round_up(ix->dim, 16));
-    CUDA_TRY(sc->q_f32.ensure(nq * qstride));
-    CUDA_TRY(sc->q_codes.ensure(nq * qstride));
-    CUDA_TRY(sc->q_aux.ensure(nq * 2));
     const bool counting = ix->counting != 0;
     if (counting) {
         CUDA_TRY(sc->hops.ensure(nq));
@@ -1199,45 +1171,25 @@ static int search_on_device(svsb200_index* ix, Replica* rep, Scratch* sc, const 
         CUDA_TRY(sc->fetched.ensure(nq));
         sc->counted_nq = nq;
     }
-
-    cudaError_t err;
-    switch (qdtype) {
-        case SVSB200_F32:
-            err = launch_prepare<SVSB200_F32>(d_queries, uint32_t(nq), uint32_t(ix->dim), qstride, mode, metric, ix->dtype,
-                                              ix->scale, ix->bias, rep->d_mean, sc->q_f32.ptr, sc->q_codes.ptr, sc->q_aux.ptr, stream);
-            break;
-        case SVSB200_F16:
-            err = launch_prepare<SVSB200_F16>(d_queries, uint32_t(nq), uint32_t(ix->dim), qstride, mode, metric, ix->dtype,
-                                              ix->scale, ix->bias, rep->d_mean, sc->q_f32.ptr, sc->q_codes.ptr, sc->q_aux.ptr, stream);
-            break;
-        case SVSB200_I8:
-            err = launch_prepare<SVSB200_I8>(d_queries, uint32_t(nq), uint32_t(ix->dim), qstride, mode, metric, ix->dtype,
-                                             ix->scale, ix->bias, rep->d_mean, sc->q_f32.ptr, sc->q_codes.ptr, sc->q_aux.ptr, stream);
-            break;
-        default:
-            err = launch_prepare<SVSB200_U8>(d_queries, uint32_t(nq), uint32_t(ix->dim), qstride, mode, metric, ix->dtype,
-                                             ix->scale, ix->bias, rep->d_mean, sc->q_f32.ptr, sc->q_codes.ptr, sc->q_aux.ptr, stream);
-    }
-    CUDA_TRY(err);
-    CUDA_TRY(cudaMemsetAsync(sc->d_counter, 0, sizeof(unsigned int), stream));
+    if (int rc = prepare_queries(ix, rep, sc, d_queries, qdtype, nq, mode, stream)) return rc;
+    CUDA_TRY(cudaMemsetAsync(sc->d_counter.ptr, 0, sizeof(unsigned int), stream));
     // (sc->d_cancel is zero here: only wait_kernels raises it, and lowers it again once the kernels have finished)
 
     SearchParams p{};
-    p.vectors = rep->d_vectors;
-    p.graph = rep->d_graph;
-    p.ref_degree = rep->d_ref_degree;
+    p.vectors = rep->d_vectors.ptr;
+    p.graph = rep->d_graph.ptr;
+    p.ref_degree = rep->d_ref_degree.ptr;
     p.n = uint32_t(ix->n);
     p.dim = uint32_t(ix->dim);
     p.row_stride = ix->row_stride;
     p.gstride = ix->gstride;
     p.entry_point = ix->entry_point;
-    p.entry_points = rep->d_entry;
+    p.entry_points = rep->d_entry.ptr;
     // push_back drops entry points once the buffer is full (search_buffer.h:311-316): only the first `capacity` count
-    p.n_entry = rep->d_entry ? uint32_t(std::min<size_t>(ix->n_entry, capacity)) : 1;
+    p.n_entry = rep->d_entry.ptr ? uint32_t(std::min<size_t>(ix->n_entry, capacity)) : 1;
     p.greater = metric != SVSB200_L2;
     p.sq = ix->storage == SVSB200_SQ;
     p.lvq = ix->storage == SVSB200_LVQ8;
-    p.no_split = int(ix->no_split);
     p.lvq_const_offset = ix->lvq_const_offset;
     p.scale = ix->scale;
     p.bias = ix->bias;
@@ -1245,7 +1197,7 @@ static int search_on_device(svsb200_index* ix, Replica* rep, Scratch* sc, const 
     p.qf = sc->q_f32.ptr;
     p.qcodes = sc->q_codes.ptr;
     p.qaux = sc->q_aux.ptr;
-    p.qstride = qstride;
+    p.qstride = qstride_for(ix->dim);
     p.nq = uint32_t(nq);
     p.k = uint32_t(k);
     p.window = uint32_t(window);
@@ -1256,8 +1208,8 @@ static int search_on_device(svsb200_index* ix, Replica* rep, Scratch* sc, const 
     p.id_bytes = id_bytes;
     p.id_offset = id_bytes == 8 ? ix->id_offset : 0;
     p.out_dists = d_out_dists;
-    p.work_counter = sc->d_counter;
-    p.cancel = sc->poll_cancel ? sc->d_cancel : nullptr;   // (no predicate: no per-hop poll in the kernel)
+    p.work_counter = sc->d_counter.ptr;
+    p.cancel = sc->poll_cancel ? sc->d_cancel.ptr : nullptr;   // (no predicate: no per-hop poll in the kernel)
     p.hops = counting ? sc->hops.ptr : nullptr;
     p.evals = counting ? sc->evals.ptr : nullptr;
     p.fetched = counting ? sc->fetched.ptr : nullptr;
@@ -1266,7 +1218,7 @@ static int search_on_device(svsb200_index* ix, Replica* rep, Scratch* sc, const 
     // below the 0xFFFF "empty" mark; larger indexes fall back to direct-mapped 32-bit entries.
     p.filter_shift = 0;
     while ((2u << p.filter_shift) < p.filter_slots) ++p.filter_shift;   // log2(sets) with sets = slots / 2
-    p.filter_tag16 = p.filter_slots >= 2 && ((uint64_t(ix->n - 1) >> p.filter_shift) < 0xFFFFull) && ix->filter_tag16 != 0;
+    p.filter_tag16 = p.filter_slots >= 2 && ((uint64_t(ix->n - 1) >> p.filter_shift) < 0xFFFFull);
     if (!p.filter_tag16) {
         p.filter_shift = 0;
         while ((1u << p.filter_shift) < p.filter_slots) ++p.filter_shift;
@@ -1276,29 +1228,21 @@ static int search_on_device(svsb200_index* ix, Replica* rep, Scratch* sc, const 
     const size_t smem_limit = 227 * 1024;
     // The lean kernel (search_fast.cuh) covers the common shape: 16-bit-tag filter on, adjacency rows of up to
     // 128 neighbours; anything else (and the exhaustive scan) runs on the generic kernel.
-    const uint32_t fast_cap_pad = uint32_t(round_up(capacity, 32));
-    // its filter: sets of eight 16-bit tags; default 256 sets (4 KB), more when n needs it for exactness
-    uint32_t fast_slots = ix->filter_slots < 0 ? 2048u : uint32_t(ix->filter_slots);
-    if (fast_slots && fast_slots < 64) fast_slots = 64;
-    uint32_t fast_shift = 0;
-    while ((8u << fast_shift) < fast_slots) ++fast_shift;                       // log2(sets)
-    while (fast_slots && (uint64_t(ix->n - 1) >> fast_shift) >= 0xFFFFull && fast_shift < 20) {
-        ++fast_shift;
-        fast_slots <<= 1;
-    }
-    const size_t fast_bytes = fast_smem_bytes(p.qstride, fast_cap_pad, p.deg_pad, fast_slots * 2u);
-    const bool use_fast = !exhaustive && !ix->generic_kernel && fast_slots >= 64 && ix->filter_tag16 &&
-                          (uint64_t(ix->n - 1) >> fast_shift) < 0xFFFFull && p.deg_pad <= 32u * kFastMaxGW &&
-                          p.gstride % 32u == 0 && fast_bytes <= smem_limit;
+    // Its filter: default 256 sets (4 KB).
+    const LeanFilterPlan fast = lean_filter_plan(ix->n, ix->dim, capacity, p.deg_pad,
+                                                 ix->filter_slots < 0 ? 2048u : uint32_t(ix->filter_slots));
+    const bool use_fast = !exhaustive && !ix->generic_kernel && fast.slots >= 64 &&
+                          (uint64_t(ix->n - 1) >> fast.shift) < 0xFFFFull && p.deg_pad <= 32u * kFastMaxGW &&
+                          p.gstride % 32u == 0 && fast.smem_bytes <= smem_limit;
     sc->last_kernel = use_fast ? 1 : 0;
     const int nrows = ix->rows_in_flight ? int(ix->rows_in_flight) : 2;
     if (use_fast) {
-        p.cap_pad = fast_cap_pad;
-        p.filter_slots = fast_slots;
-        p.filter_shift = fast_shift;
+        p.cap_pad = uint32_t(round_up(capacity, 32));
+        p.filter_slots = fast.slots;
+        p.filter_shift = fast.shift;
         p.filter_tag16 = 1;
         cfg.warps_per_cta = 1;
-        cfg.smem_bytes = fast_bytes;
+        cfg.smem_bytes = fast.smem_bytes;
         cfg.stream = stream;
         cfg.grid = ix->ctas_per_sm ? rep->sm_count * int(ix->ctas_per_sm) : -rep->sm_count;
     } else {
@@ -1317,6 +1261,7 @@ static int search_on_device(svsb200_index* ix, Replica* rep, Scratch* sc, const 
 
     CUDA_TRY(cudaEventRecord(sc->ev_start, stream));
     const int rowt = ix->storage == SVSB200_LVQ8 ? ROW_LVQ8 : ix->dtype;
+    cudaError_t err;
     if (exhaustive) {
         // few queries: cut the base rows into ranges so that (query, range) work items fill the GPU; the per-range
         // top-k lists are merged with TotalOrder (== the scan's own order: key, then id)
@@ -1330,37 +1275,14 @@ static int search_on_device(svsb200_index* ix, Replica* rep, Scratch* sc, const 
             p.out_dists = sc->exh_dists.ptr;
             p.exh_split = split;
         }
-        switch (rowt) {
-            case ROW_LVQ8: err = launch_search_exhaustive<ROW_LVQ8>(op, p, cfg); break;
-            case SVSB200_F32: err = launch_search_exhaustive<SVSB200_F32>(op, p, cfg); break;
-            case SVSB200_F16: err = launch_search_exhaustive<SVSB200_F16>(op, p, cfg); break;
-            case SVSB200_I8: err = launch_search_exhaustive<SVSB200_I8>(op, p, cfg); break;
-            default: err = launch_search_exhaustive<SVSB200_U8>(op, p, cfg);
-        }
-        if (err == cudaSuccess && split > 1) {
-            const unsigned warps = 4;
-            merge_topk_kernel<<<unsigned((nq + warps - 1) / warps), warps * 32, 0, stream>>>(
-                sc->exh_ids.ptr, sc->exh_dists.ptr, split, uint32_t(nq), uint32_t(k), metric != SVSB200_L2,
-                static_cast<uint64_t*>(d_out_ids), d_out_dists);
-            count_launch();
-            err = cudaGetLastError();
-        }
+        err = with_row_type(rowt, [&](auto t) { return launch_search_exhaustive<decltype(t)::value>(op, p, cfg); });
+        if (err == cudaSuccess && split > 1)
+            err = launch_merge_topk(sc->exh_ids.ptr, sc->exh_dists.ptr, split, nq, k, metric != SVSB200_L2,
+                                    static_cast<uint64_t*>(d_out_ids), d_out_dists, stream);
     } else if (use_fast) {
-        switch (rowt) {
-            case ROW_LVQ8: err = launch_search_fast<ROW_LVQ8>(op, p, cfg); break;
-            case SVSB200_F32: err = launch_search_fast<SVSB200_F32>(op, p, cfg); break;
-            case SVSB200_F16: err = launch_search_fast<SVSB200_F16>(op, p, cfg); break;
-            case SVSB200_I8: err = launch_search_fast<SVSB200_I8>(op, p, cfg); break;
-            default: err = launch_search_fast<SVSB200_U8>(op, p, cfg);
-        }
+        err = with_row_type(rowt, [&](auto t) { return launch_search_fast<decltype(t)::value>(op, p, cfg); });
     } else {
-        switch (rowt) {
-            case ROW_LVQ8: err = launch_search<ROW_LVQ8>(op, p, cfg, nrows); break;
-            case SVSB200_F32: err = launch_search<SVSB200_F32>(op, p, cfg, nrows); break;
-            case SVSB200_F16: err = launch_search<SVSB200_F16>(op, p, cfg, nrows); break;
-            case SVSB200_I8: err = launch_search<SVSB200_I8>(op, p, cfg, nrows); break;
-            default: err = launch_search<SVSB200_U8>(op, p, cfg, nrows);
-        }
+        err = with_row_type(rowt, [&](auto t) { return launch_search<decltype(t)::value>(op, p, cfg, nrows); });
     }
     CUDA_TRY(err);
     CUDA_TRY(cudaEventRecord(sc->ev_stop, stream));
@@ -1378,27 +1300,23 @@ int svsb200_search_device(svsb200_index* ix, const void* d_queries, int qdtype, 
     (void)use_visited_set;   // performance-only in the reference (search_buffer.h:420); results identical
     if (!ix) return fail("svsb200_search_device: NULL index");
     if (nq && (!d_queries || !d_out_ids || !d_out_dists)) return fail("svsb200_search_device: NULL buffer");
-    if (ix->reps.size() != 1) return fail("svsb200_search_device: the index must live on exactly one device");
-    Replica* rep = ix->reps[0].get();
-    CUDA_TRY(cudaSetDevice(rep->device));
-    std::string err;
-    // NULL = the stream of a scratch this index keeps for that purpose (ordered against itself)
-    Scratch* sc = scratch_for_stream(rep, static_cast<cudaStream_t>(stream_), &err);
-    if (!sc) return fail(err);
-    return search_on_device(ix, rep, sc, d_queries, qdtype, nq, k, window, capacity, d_out_ids, id_bytes, d_out_dists,
+    Scratch* sc = nullptr;
+    if (int rc = device_api_scratch("svsb200_search_device", ix, stream_, &sc)) return rc;
+    return search_on_device(ix, ix->reps[0].get(), sc, d_queries, qdtype, nq, k, window, capacity, d_out_ids, id_bytes, d_out_dists,
                             sc->stream);
 }
 
 // Waits for the search kernels of `scs` (their ev_stop events); with a cancel callback it polls the callback
 // meanwhile and raises the device flags the kernels poll per query and per hop (greedy_search.h:155,
 // extensions.h:579).
-static int wait_kernels(const std::vector<Scratch*>& scs, int (*cancel)(void*), void* cancel_arg) {
+static int wait_kernels(const std::vector<ScratchLease>& scs, int (*cancel)(void*), void* cancel_arg) {
     if (!cancel) return 0;   // nothing to poll for: the stream order of the copies behind the kernels is enough
     bool raised = false;
     int rc = 0;
     for (;;) {
         bool busy = false;
-        for (Scratch* sc : scs) {
+        for (const ScratchLease& l : scs) {
+            Scratch* sc = l.sc;
             if (!sc->timed) continue;
             cudaSetDevice(sc->device);
             cudaError_t q = cudaEventQuery(sc->ev_stop);
@@ -1408,28 +1326,28 @@ static int wait_kernels(const std::vector<Scratch*>& scs, int (*cancel)(void*), 
         if (!busy || rc) break;
         if (!raised && cancel(cancel_arg)) {
             raised = true;
-            for (Scratch* sc : scs) {
-                cudaSetDevice(sc->device);
-                cudaError_t e = cudaMemsetAsync(sc->d_cancel, 1, sizeof(int), sc->ctl);
+            for (const ScratchLease& l : scs) {
+                cudaSetDevice(l.sc->device);
+                cudaError_t e = cudaMemsetAsync(l.sc->d_cancel.ptr, 1, sizeof(int), l.sc->ctl);
                 if (e != cudaSuccess) rc = fail(std::string("cudaMemsetAsync: ") + cudaGetErrorString(e));
             }
         }
         std::this_thread::sleep_for(std::chrono::microseconds(20));
     }
     if (raised) {   // the kernels are done (or failed): lower the flags for the next search of these scratch sets
-        for (Scratch* sc : scs) {
-            cudaSetDevice(sc->device);
-            cudaStreamSynchronize(sc->stream);
-            cudaMemsetAsync(sc->d_cancel, 0, sizeof(int), sc->ctl);
-            cudaStreamSynchronize(sc->ctl);
+        for (const ScratchLease& l : scs) {
+            cudaSetDevice(l.sc->device);
+            cudaStreamSynchronize(l.sc->stream);
+            cudaMemsetAsync(l.sc->d_cancel.ptr, 0, sizeof(int), l.sc->ctl);
+            cudaStreamSynchronize(l.sc->ctl);
         }
     }
     return rc;
 }
-static int wait_all(const std::vector<Scratch*>& scs) {
-    for (Scratch* sc : scs) {
-        cudaSetDevice(sc->device);
-        CUDA_TRY(cudaStreamSynchronize(sc->stream));
+static int wait_all(const std::vector<ScratchLease>& scs) {
+    for (const ScratchLease& l : scs) {
+        cudaSetDevice(l.sc->device);
+        CUDA_TRY(cudaStreamSynchronize(l.sc->stream));
     }
     return 0;
 }
@@ -1447,8 +1365,7 @@ int svsb200_search_cancellable(svsb200_index* ix, const void* queries, int qdtyp
     if (stream_ && R != 1) return fail("svsb200_search: a caller stream needs a single-device index");
     if (cancel && cancel(cancel_arg)) return 0;   // index.h:575 checks before any work
     const size_t qrow = ix->dim * esize(qdtype);
-    std::vector<Scratch*> used;
-    std::vector<Replica*> used_rep;
+    std::vector<ScratchLease> used;
     std::vector<size_t> used_lo, used_m;
     int rc = 0;
     // Every device's share is cut into C pieces, each on its own stream: the host-to-device copy of piece i+1 and the
@@ -1469,19 +1386,10 @@ int svsb200_search_cancellable(svsb200_index* ix, const void* queries, int qdtyp
         balance(nq, R * C, part, &lo, &hi);
         if (hi == lo) continue;
         Replica* rep = ix->reps[r].get();
-        cudaError_t e = cudaSetDevice(rep->device);
-        if (e != cudaSuccess) {
-            rc = fail(std::string("cudaSetDevice: ") + cudaGetErrorString(e));
-            break;
-        }
-        std::string err;
-        Scratch* sc = stream_ ? scratch_for_stream(rep, static_cast<cudaStream_t>(stream_), &err) : acquire(rep, &err);
-        if (!sc) {
-            rc = fail(err);
-            break;
-        }
-        used.push_back(sc);
-        used_rep.push_back(stream_ ? nullptr : rep);
+        ScratchLease lease;
+        if ((rc = lease.take(rep, static_cast<cudaStream_t>(stream_)))) break;
+        Scratch* sc = lease.sc;
+        used.push_back(std::move(lease));
         const size_t m = hi - lo;
         used_lo.push_back(lo);
         used_m.push_back(m);
@@ -1493,9 +1401,8 @@ int svsb200_search_cancellable(svsb200_index* ix, const void* queries, int qdtyp
             CUDA_TRY(sc->dists.ensure(m * k));
             CUDA_TRY(cudaMemcpyAsync(sc->q_raw.ptr, static_cast<const char*>(queries) + lo * qrow, m * qrow,
                                      cudaMemcpyHostToDevice, sc->stream));
-            int rc2 = search_on_device(ix, rep, sc, sc->q_raw.ptr, qdtype, m, k, window, capacity, sc->ids.ptr, id_bytes,
-                                       sc->dists.ptr, sc->stream);
-            return rc2;
+            return search_on_device(ix, rep, sc, sc->q_raw.ptr, qdtype, m, k, window, capacity, sc->ids.ptr, id_bytes,
+                                    sc->dists.ptr, sc->stream);
         };
         rc = step();
     }
@@ -1504,7 +1411,7 @@ int svsb200_search_cancellable(svsb200_index* ix, const void* queries, int qdtyp
     // memory would block this thread, so the device-to-host copies are only enqueued afterwards)
     int rc_wait = wait_kernels(used, cancel, cancel_arg);
     for (size_t i = 0; i < used.size() && rc == 0 && rc_wait == 0; ++i) {
-        Scratch* sc = used[i];
+        Scratch* sc = used[i].sc;
         if (!sc->timed) continue;
         auto copy_out = [&]() -> int {
             CUDA_TRY(cudaSetDevice(sc->device));
@@ -1518,10 +1425,7 @@ int svsb200_search_cancellable(svsb200_index* ix, const void* queries, int qdtyp
         if (rc) first_error = g_error;
     }
     if (rc_wait == 0) rc_wait = wait_all(used);
-    for (size_t i = 0; i < used.size(); ++i) {
-        used[i]->poll_cancel = false;
-        if (used_rep[i]) release(used_rep[i], used[i]);
-    }
+    for (const ScratchLease& l : used) l.sc->poll_cancel = false;
     if (rc) {
         g_error = first_error;
         return rc;
@@ -1535,14 +1439,30 @@ int svsb200_search(svsb200_index* ix, const void* queries, int qdtype, size_t nq
                                       out_dists, stream_, nullptr, nullptr);
 }
 
-// Runs the batch with a result list of `kk` entries per query (window = capacity = max(window, kk)) into the scratch's
-// own id / distance blocks.
-static int search_long_lists(svsb200_index* ix, Replica* rep, Scratch* sc, const void* d_queries, int qdtype, size_t nq, size_t kk,
-                             size_t window) {
-    CUDA_TRY(sc->ids.ensure(nq * kk * 8));
-    CUDA_TRY(sc->dists.ensure(nq * kk));
-    const size_t w = std::max(window, kk);
-    return search_on_device(ix, rep, sc, d_queries, qdtype, nq, kk, w, w, sc->ids.ptr, 8, sc->dists.ptr, sc->stream);
+// Searches the queries in sc->q_raw with result lists of `kk` entries (window = capacity = max(window, kk)) into the
+// scratch's own id / distance blocks; `check(kk)` enqueues the kernel that counts the queries that need longer lists
+// into *d_unfinished.  The lists grow (x4) until no query is unfinished, like the reference's batch iterator asks for
+// further batches (vamana_index_impl.h:183-205).  *kk is the length of the last lists.
+extern "C++" template <typename Check>
+int search_growing_lists(svsb200_index* ix, Replica* rep, Scratch* sc, int qdtype, size_t nq, size_t window,
+                         uint32_t* d_unfinished, size_t* kk, Check check) {
+    for (;;) {
+        *kk = std::min(*kk, ix->n);
+        CUDA_TRY(sc->ids.ensure(nq * *kk * 8));
+        CUDA_TRY(sc->dists.ensure(nq * *kk));
+        const size_t w = std::max(window, *kk);
+        int rc = search_on_device(ix, rep, sc, sc->q_raw.ptr, qdtype, nq, *kk, w, w, sc->ids.ptr, 8, sc->dists.ptr, sc->stream);
+        if (rc) return rc;
+        CUDA_TRY(cudaMemsetAsync(d_unfinished, 0, 4, sc->stream));
+        check(*kk);
+        count_launch();
+        CUDA_TRY(cudaGetLastError());
+        uint32_t unfinished = 0;
+        CUDA_TRY(cudaMemcpyAsync(&unfinished, d_unfinished, 4, cudaMemcpyDeviceToHost, sc->stream));
+        CUDA_TRY(cudaStreamSynchronize(sc->stream));
+        if (unfinished == 0 || *kk >= ix->n || *kk >= 16384) return 0;
+        *kk *= 4;
+    }
 }
 
 int svsb200_search_filtered(svsb200_index* ix, const void* queries, int qdtype, size_t nq, size_t k, size_t window,
@@ -1553,64 +1473,43 @@ int svsb200_search_filtered(svsb200_index* ix, const void* queries, int qdtype, 
     if (k == 0) return fail("k must be greater than 0");
     if (qdtype < SVSB200_F32 || qdtype > SVSB200_U8) return fail("bad query dtype");
     Replica* rep = ix->reps[0].get();
-    CUDA_TRY(cudaSetDevice(rep->device));
-    std::string err;
-    Scratch* sc = acquire(rep, &err);
-    if (!sc) return fail(err);
-    uint32_t *d_bitmap = nullptr, *d_found = nullptr;
-    uint64_t* d_oi = nullptr;
-    float* d_od = nullptr;
-    auto body = [&]() -> int {
-        const size_t words = (ix->n + 31) / 32;
-        const size_t qbytes = nq * ix->dim * esize(qdtype);
-        CUDA_TRY(cudaMalloc(&d_bitmap, words * 4));
-        CUDA_TRY(cudaMalloc(&d_found, (nq + 1) * 4));
-        CUDA_TRY(cudaMalloc(&d_oi, nq * k * 8));
-        CUDA_TRY(cudaMalloc(&d_od, nq * k * 4));
-        CUDA_TRY(sc->q_raw.ensure(qbytes));
-        CUDA_TRY(cudaMemcpyAsync(d_bitmap, id_bitmap, words * 4, cudaMemcpyHostToDevice, sc->stream));
-        CUDA_TRY(cudaMemcpyAsync(sc->q_raw.ptr, queries, qbytes, cudaMemcpyHostToDevice, sc->stream));
-        CUDA_TRY(cudaMemsetAsync(d_oi, 0xFF, nq * k * 8, sc->stream));
-        // lists grow (x4) until every query has k members or its search is exhausted, like the reference's batch
-        // iterator asks for further batches (vamana_index_impl.h:183-205)
-        size_t kk = std::max(k, window);
-        for (;;) {
-            kk = std::min(kk, ix->n);
-            int rc = search_long_lists(ix, rep, sc, sc->q_raw.ptr, qdtype, nq, kk, window);
-            if (rc) return rc;
-            CUDA_TRY(cudaMemsetAsync(d_found + nq, 0, 4, sc->stream));
-            filter_topk_kernel<<<unsigned((nq + 3) / 4), 128, 0, sc->stream>>>(
-                reinterpret_cast<const uint64_t*>(sc->ids.ptr), sc->dists.ptr, uint32_t(nq), uint32_t(kk), uint32_t(k), d_bitmap,
-                d_oi, d_od, d_found, d_found + nq);
-            count_launch();
-            CUDA_TRY(cudaGetLastError());
-            uint32_t unfinished = 0;
-            CUDA_TRY(cudaMemcpyAsync(&unfinished, d_found + nq, 4, cudaMemcpyDeviceToHost, sc->stream));
-            CUDA_TRY(cudaStreamSynchronize(sc->stream));
-            if (unfinished == 0 || kk >= ix->n || kk >= 16384) break;
-            kk *= 4;
+    ScratchLease lease;   // (declared first: returned after the buffers below are freed)
+    if (int rc = lease.take(rep, nullptr)) return rc;
+    Scratch* sc = lease.sc;
+    DeviceBuffer<uint32_t> d_bitmap, d_found;
+    DeviceBuffer<uint64_t> d_oi;
+    DeviceBuffer<float> d_od;
+    const size_t words = (ix->n + 31) / 32;
+    const size_t qbytes = nq * ix->dim * esize(qdtype);
+    CUDA_TRY(d_bitmap.ensure(words));
+    CUDA_TRY(d_found.ensure(nq + 1));
+    CUDA_TRY(d_oi.ensure(nq * k));
+    CUDA_TRY(d_od.ensure(nq * k));
+    CUDA_TRY(sc->q_raw.ensure(qbytes));
+    CUDA_TRY(cudaMemcpyAsync(d_bitmap.ptr, id_bitmap, words * 4, cudaMemcpyHostToDevice, sc->stream));
+    CUDA_TRY(cudaMemcpyAsync(sc->q_raw.ptr, queries, qbytes, cudaMemcpyHostToDevice, sc->stream));
+    CUDA_TRY(cudaMemsetAsync(d_oi.ptr, 0xFF, nq * k * 8, sc->stream));
+    // lists grow until every query has k members or its search is exhausted
+    size_t kk = std::max(k, window);
+    int rc = search_growing_lists(ix, rep, sc, qdtype, nq, window, d_found.ptr + nq, &kk, [&](size_t len) {
+        filter_topk_kernel<<<unsigned((nq + 3) / 4), 128, 0, sc->stream>>>(
+            reinterpret_cast<const uint64_t*>(sc->ids.ptr), sc->dists.ptr, uint32_t(nq), uint32_t(len), uint32_t(k),
+            d_bitmap.ptr, d_oi.ptr, d_od.ptr, d_found.ptr, d_found.ptr + nq);
+    });
+    if (rc) return rc;
+    std::vector<uint32_t> found(nq);
+    CUDA_TRY(cudaMemcpyAsync(found.data(), d_found.ptr, nq * 4, cudaMemcpyDeviceToHost, sc->stream));
+    CUDA_TRY(cudaMemcpyAsync(out_ids, d_oi.ptr, nq * k * 8, cudaMemcpyDeviceToHost, sc->stream));
+    CUDA_TRY(cudaMemcpyAsync(out_dists, d_od.ptr, nq * k * 4, cudaMemcpyDeviceToHost, sc->stream));
+    CUDA_TRY(cudaStreamSynchronize(sc->stream));
+    for (size_t q = 0; q < nq; ++q) {   // pad like the reference: unspecified id (all-ones), +inf distance
+        for (size_t j = found[q]; j < k; ++j) {
+            out_ids[q * k + j] = ~uint64_t(0);
+            out_dists[q * k + j] = INFINITY;
         }
-        std::vector<uint32_t> found(nq);
-        CUDA_TRY(cudaMemcpyAsync(found.data(), d_found, nq * 4, cudaMemcpyDeviceToHost, sc->stream));
-        CUDA_TRY(cudaMemcpyAsync(out_ids, d_oi, nq * k * 8, cudaMemcpyDeviceToHost, sc->stream));
-        CUDA_TRY(cudaMemcpyAsync(out_dists, d_od, nq * k * 4, cudaMemcpyDeviceToHost, sc->stream));
-        CUDA_TRY(cudaStreamSynchronize(sc->stream));
-        for (size_t q = 0; q < nq; ++q) {   // pad like the reference: unspecified id (all-ones), +inf distance
-            for (size_t j = found[q]; j < k; ++j) {
-                out_ids[q * k + j] = ~uint64_t(0);
-                out_dists[q * k + j] = INFINITY;
-            }
-            if (out_found) out_found[q] = found[q];
-        }
-        return 0;
-    };
-    int rc = body();
-    if (d_bitmap) cudaFree(d_bitmap);
-    if (d_found) cudaFree(d_found);
-    if (d_oi) cudaFree(d_oi);
-    if (d_od) cudaFree(d_od);
-    release(rep, sc);
-    return rc;
+        if (out_found) out_found[q] = found[q];
+    }
+    return 0;
 }
 
 int svsb200_range_search(svsb200_index* ix, const void* queries, int qdtype, size_t nq, float radius, size_t window,
@@ -1622,62 +1521,46 @@ int svsb200_range_search(svsb200_index* ix, const void* queries, int qdtype, siz
     *out_ids = nullptr;
     *out_dists = nullptr;
     Replica* rep = ix->reps[0].get();
-    CUDA_TRY(cudaSetDevice(rep->device));
-    std::string err;
-    Scratch* sc = acquire(rep, &err);
-    if (!sc) return fail(err);
-    uint32_t* d_counts = nullptr;
-    auto body = [&]() -> int {
-        const size_t qbytes = nq * ix->dim * esize(qdtype);
-        CUDA_TRY(cudaMalloc(&d_counts, (nq + 1) * 4));
-        CUDA_TRY(sc->q_raw.ensure(qbytes));
-        CUDA_TRY(cudaMemcpyAsync(sc->q_raw.ptr, queries, qbytes, cudaMemcpyHostToDevice, sc->stream));
-        size_t kk = std::max<size_t>(window, 16);
-        for (;;) {
-            kk = std::min(kk, ix->n);
-            int rc = search_long_lists(ix, rep, sc, sc->q_raw.ptr, qdtype, nq, kk, window);
-            if (rc) return rc;
-            CUDA_TRY(cudaMemsetAsync(d_counts + nq, 0, 4, sc->stream));
-            range_count_kernel<<<unsigned((nq + 127) / 128), 128, 0, sc->stream>>>(
-                sc->dists.ptr, reinterpret_cast<const uint64_t*>(sc->ids.ptr), uint32_t(nq), uint32_t(kk), radius,
-                ix->metric != SVSB200_L2, d_counts, d_counts + nq);
-            count_launch();
-            CUDA_TRY(cudaGetLastError());
-            uint32_t unfinished = 0;
-            CUDA_TRY(cudaMemcpyAsync(&unfinished, d_counts + nq, 4, cudaMemcpyDeviceToHost, sc->stream));
-            CUDA_TRY(cudaStreamSynchronize(sc->stream));
-            if (unfinished == 0 || kk >= ix->n || kk >= 16384) break;
-            kk *= 4;
+    ScratchLease lease;   // (declared first: returned after the buffer below is freed)
+    if (int rc = lease.take(rep, nullptr)) return rc;
+    Scratch* sc = lease.sc;
+    DeviceBuffer<uint32_t> d_counts;
+    const size_t qbytes = nq * ix->dim * esize(qdtype);
+    CUDA_TRY(d_counts.ensure(nq + 1));
+    CUDA_TRY(sc->q_raw.ensure(qbytes));
+    CUDA_TRY(cudaMemcpyAsync(sc->q_raw.ptr, queries, qbytes, cudaMemcpyHostToDevice, sc->stream));
+    // lists grow until every query's last result lies outside the radius or its search is exhausted
+    size_t kk = std::max<size_t>(window, 16);
+    int rc = search_growing_lists(ix, rep, sc, qdtype, nq, window, d_counts.ptr + nq, &kk, [&](size_t len) {
+        range_count_kernel<<<unsigned((nq + 127) / 128), 128, 0, sc->stream>>>(
+            sc->dists.ptr, reinterpret_cast<const uint64_t*>(sc->ids.ptr), uint32_t(nq), uint32_t(len), radius,
+            ix->metric != SVSB200_L2, d_counts.ptr, d_counts.ptr + nq);
+    });
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(out_counts, d_counts.ptr, nq * 4, cudaMemcpyDeviceToHost, sc->stream));
+    std::vector<uint64_t> ids(nq * kk);
+    std::vector<float> dd(nq * kk);
+    CUDA_TRY(cudaMemcpyAsync(ids.data(), sc->ids.ptr, nq * kk * 8, cudaMemcpyDeviceToHost, sc->stream));
+    CUDA_TRY(cudaMemcpyAsync(dd.data(), sc->dists.ptr, nq * kk * 4, cudaMemcpyDeviceToHost, sc->stream));
+    CUDA_TRY(cudaStreamSynchronize(sc->stream));
+    size_t total = 0;
+    for (size_t q = 0; q < nq; ++q) total += out_counts[q];
+    uint64_t* oi = static_cast<uint64_t*>(malloc(std::max<size_t>(total, 1) * 8));
+    float* od = static_cast<float*>(malloc(std::max<size_t>(total, 1) * 4));
+    if (!oi || !od) {
+        free(oi);
+        free(od);
+        return fail("svsb200_range_search: out of host memory");
+    }
+    size_t o = 0;
+    for (size_t q = 0; q < nq; ++q)
+        for (size_t j = 0; j < out_counts[q]; ++j, ++o) {
+            oi[o] = ids[q * kk + j];
+            od[o] = dd[q * kk + j];
         }
-        CUDA_TRY(cudaMemcpyAsync(out_counts, d_counts, nq * 4, cudaMemcpyDeviceToHost, sc->stream));
-        std::vector<uint64_t> ids(nq * kk);
-        std::vector<float> dd(nq * kk);
-        CUDA_TRY(cudaMemcpyAsync(ids.data(), sc->ids.ptr, nq * kk * 8, cudaMemcpyDeviceToHost, sc->stream));
-        CUDA_TRY(cudaMemcpyAsync(dd.data(), sc->dists.ptr, nq * kk * 4, cudaMemcpyDeviceToHost, sc->stream));
-        CUDA_TRY(cudaStreamSynchronize(sc->stream));
-        size_t total = 0;
-        for (size_t q = 0; q < nq; ++q) total += out_counts[q];
-        uint64_t* oi = static_cast<uint64_t*>(malloc(std::max<size_t>(total, 1) * 8));
-        float* od = static_cast<float*>(malloc(std::max<size_t>(total, 1) * 4));
-        if (!oi || !od) {
-            free(oi);
-            free(od);
-            return fail("svsb200_range_search: out of host memory");
-        }
-        size_t o = 0;
-        for (size_t q = 0; q < nq; ++q)
-            for (size_t j = 0; j < out_counts[q]; ++j, ++o) {
-                oi[o] = ids[q * kk + j];
-                od[o] = dd[q * kk + j];
-            }
-        *out_ids = oi;
-        *out_dists = od;
-        return 0;
-    };
-    int rc = body();
-    if (d_counts) cudaFree(d_counts);
-    release(rep, sc);
-    return rc;
+    *out_ids = oi;
+    *out_dists = od;
+    return 0;
 }
 
 void svsb200_free(void* p) { free(p); }
@@ -1696,24 +1579,13 @@ int svsb200_search_sharded(svsb200_index* const* shards, size_t nshards, const v
     }
     const size_t qbytes = nq * shards[0]->dim * esize(qdtype);
     const size_t cnt = nq * k;
-    std::vector<Scratch*> scs(nshards, nullptr);
-    std::string err;
-    auto give_back = [&]() {
-        for (size_t s = 0; s < nshards; ++s)
-            if (scs[s]) release(shards[s]->reps[0].get(), scs[s]);
-    };
+    std::vector<ScratchLease> scs(nshards);
     for (size_t s = 0; s < nshards; ++s) {
-        Replica* rep = shards[s]->reps[0].get();
-        cudaSetDevice(rep->device);
-        scs[s] = acquire(rep, &err);
-        if (!scs[s]) {
-            give_back();
-            return fail(err);
-        }
+        if (int rc = scs[s].take(shards[s]->reps[0].get(), nullptr)) return rc;
     }
     // the merging device is shard 0's; its scratch holds the [nshards][nq][k] gather block
     Replica* rep0 = shards[0]->reps[0].get();
-    Scratch* sc0 = scs[0];
+    Scratch* sc0 = scs[0].sc;
     auto body = [&]() -> int {
         CUDA_TRY(cudaSetDevice(rep0->device));
         CUDA_TRY(sc0->gather_ids.ensure(nshards * cnt));
@@ -1722,7 +1594,7 @@ int svsb200_search_sharded(svsb200_index* const* shards, size_t nshards, const v
         CUDA_TRY(sc0->merged_dists.ensure(cnt));
         for (size_t s = 0; s < nshards; ++s) {
             Replica* rep = shards[s]->reps[0].get();
-            Scratch* sc = scs[s];
+            Scratch* sc = scs[s].sc;
             CUDA_TRY(cudaSetDevice(rep->device));
             CUDA_TRY(sc->q_raw.ensure(qbytes));
             CUDA_TRY(cudaMemcpyAsync(sc->q_raw.ptr, queries, qbytes, cudaMemcpyHostToDevice, sc->stream));
@@ -1759,12 +1631,8 @@ int svsb200_search_sharded(svsb200_index* const* shards, size_t nshards, const v
             }
         }
         CUDA_TRY(cudaSetDevice(rep0->device));
-        const unsigned warps = 4;
-        merge_topk_kernel<<<unsigned((nq + warps - 1) / warps), warps * 32, 0, sc0->stream>>>(
-            sc0->gather_ids.ptr, sc0->gather_dists.ptr, uint32_t(nshards), uint32_t(nq), uint32_t(k),
-            shards[0]->metric != SVSB200_L2, sc0->merged_ids.ptr, sc0->merged_dists.ptr);
-        count_launch();
-        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(launch_merge_topk(sc0->gather_ids.ptr, sc0->gather_dists.ptr, nshards, nq, k, shards[0]->metric != SVSB200_L2,
+                                   sc0->merged_ids.ptr, sc0->merged_dists.ptr, sc0->stream));
         CUDA_TRY(cudaMemcpyAsync(out_ids, sc0->merged_ids.ptr, cnt * 8, cudaMemcpyDeviceToHost, sc0->stream));
         CUDA_TRY(cudaMemcpyAsync(out_dists, sc0->merged_dists.ptr, cnt * 4, cudaMemcpyDeviceToHost, sc0->stream));
         return 0;
@@ -1772,7 +1640,6 @@ int svsb200_search_sharded(svsb200_index* const* shards, size_t nshards, const v
     int rc = body();
     const std::string first_error = g_error;
     int rc_wait = wait_all(scs);
-    give_back();
     if (rc) {
         g_error = first_error;
         return rc;
@@ -1821,11 +1688,8 @@ int svsb200_merge_topk_device(const uint64_t* d_ids, const float* d_dists, size_
     if (nshards == 0 || nshards > 1024) return fail("svsb200_merge_topk_device: 1..1024 shards supported");
     if (nq == 0 || k == 0) return 0;
     CUDA_TRY(cudaSetDevice(device));
-    const unsigned warps = 4;
-    merge_topk_kernel<<<unsigned((nq + warps - 1) / warps), warps * 32, 0, static_cast<cudaStream_t>(stream)>>>(
-        d_ids, d_dists, uint32_t(nshards), uint32_t(nq), uint32_t(k), metric != SVSB200_L2, d_out_ids, d_out_dists);
-    count_launch();
-    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(launch_merge_topk(d_ids, d_dists, nshards, nq, k, metric != SVSB200_L2, d_out_ids, d_out_dists,
+                               static_cast<cudaStream_t>(stream)));
     return 0;
 }
 
@@ -1837,26 +1701,20 @@ int svsb200_lvq8_compress(const float* data, size_t n, size_t dim, const float* 
     if (svsb200_device_count() == 0) return fail("svsb200_lvq8_compress: no CUDA device (there is no CPU fallback)");
     CUDA_TRY(cudaSetDevice(device));
     const size_t stride = svsb200_lvq8_row_stride(dim);
-    float *d_data = nullptr, *d_mean = nullptr;
-    uint8_t* d_rows = nullptr;
-    cudaError_t err = cudaMalloc(&d_data, n * dim * sizeof(float));
-    if (err == cudaSuccess) err = cudaMalloc(&d_mean, dim * sizeof(float));
-    if (err == cudaSuccess) err = cudaMalloc(&d_rows, n * stride);
-    if (err == cudaSuccess) err = cudaMemcpy(d_data, data, n * dim * sizeof(float), cudaMemcpyHostToDevice);
-    if (err == cudaSuccess) err = cudaMemcpy(d_mean, mean, dim * sizeof(float), cudaMemcpyHostToDevice);
-    if (err == cudaSuccess) {
-        const int warps = 8;
-        lvq8_compress_kernel<<<unsigned((n + warps - 1) / warps), warps * 32>>>(d_data, uint32_t(n), uint32_t(dim), d_mean,
-                                                                              d_rows, uint32_t(stride),
-                                                                              uint32_t(round_up(dim, 4)));
-        count_launch();
-        err = cudaGetLastError();
-    }
-    if (err == cudaSuccess) err = cudaMemcpy(out_rows, d_rows, n * stride, cudaMemcpyDeviceToHost);
-    if (d_data) cudaFree(d_data);
-    if (d_mean) cudaFree(d_mean);
-    if (d_rows) cudaFree(d_rows);
-    CUDA_TRY(err);
+    DeviceBuffer<float> d_data, d_mean;
+    DeviceBuffer<uint8_t> d_rows;
+    CUDA_TRY(d_data.ensure(n * dim));
+    CUDA_TRY(d_mean.ensure(dim));
+    CUDA_TRY(d_rows.ensure(n * stride));
+    CUDA_TRY(cudaMemcpy(d_data.ptr, data, n * dim * sizeof(float), cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMemcpy(d_mean.ptr, mean, dim * sizeof(float), cudaMemcpyHostToDevice));
+    const int warps = 8;
+    lvq8_compress_kernel<<<unsigned((n + warps - 1) / warps), warps * 32>>>(d_data.ptr, uint32_t(n), uint32_t(dim), d_mean.ptr,
+                                                                          d_rows.ptr, uint32_t(stride),
+                                                                          uint32_t(round_up(dim, 4)));
+    count_launch();
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaMemcpy(out_rows, d_rows.ptr, n * stride, cudaMemcpyDeviceToHost));
     return 0;
 }
 
@@ -1879,13 +1737,13 @@ static int flat_on_device(svsb200_index* ix, Replica* rep, Scratch* sc, const vo
     const int l2 = ix->metric == SVSB200_L2;
     {   // base tiles, once per replica
         std::lock_guard<std::mutex> lock(rep->mu);
-        if (!rep->flat_b) {
-            CUDA_TRY(cudaMalloc(&rep->flat_b, size_t(ntiles) * 256 * KB * 32 * 2));
-            CUDA_TRY(cudaMalloc(&rep->flat_bias, size_t(ntiles) * 256 * 4));
-            CUDA_TRY(cudaMalloc(&rep->flat_xmax, 4));
-            CUDA_TRY(cudaMemsetAsync(rep->flat_xmax, 0, 4, stream));
-            CUDA_TRY(flat_tile_rows(ix->dtype, rep->d_vectors, ix->row_stride, n, dim, 256, 1.0f, l2, rep->flat_b, rep->flat_bias,
-                                    nullptr, rep->flat_xmax, stream));
+        if (!rep->flat_b.ptr) {
+            CUDA_TRY(rep->flat_b.ensure(size_t(ntiles) * 256 * KB * 32 * 2));
+            CUDA_TRY(rep->flat_bias.ensure(size_t(ntiles) * 256));
+            CUDA_TRY(rep->flat_xmax.ensure(1));
+            CUDA_TRY(cudaMemsetAsync(rep->flat_xmax.ptr, 0, 4, stream));
+            CUDA_TRY(flat_tile_rows(ix->dtype, rep->d_vectors.ptr, ix->row_stride, n, dim, 256, 1.0f, l2, rep->flat_b.ptr,
+                                    rep->flat_bias.ptr, nullptr, rep->flat_xmax.ptr, stream));
             CUDA_TRY(cudaStreamSynchronize(stream));
         }
     }
@@ -1902,21 +1760,12 @@ static int flat_on_device(svsb200_index* ix, Replica* rep, Scratch* sc, const vo
     CUDA_TRY(cudaMemsetAsync(sc->flat_progress.ptr, 0, size_t(flat_ctas) * 4, stream));
     CUDA_TRY(flat_tile_rows(qdtype, d_queries, uint32_t(qrow), uint32_t(nq), dim, 128, 1.0f, 0, sc->flat_a.ptr, nullptr,
                             sc->flat_qnorm.ptr, nullptr, stream));
-    CUDA_TRY(flat_gemm_topk(sc->flat_a.ptr, rep->flat_b, rep->flat_bias, KB, ntiles, mtiles, flat_ctas, flat_share, nsplit, l2 ? -2.0f : -1.0f,
+    CUDA_TRY(flat_gemm_topk(sc->flat_a.ptr, rep->flat_b.ptr, rep->flat_bias.ptr, KB, ntiles, mtiles, flat_ctas, flat_share, nsplit, l2 ? -2.0f : -1.0f,
                             sc->flat_ckey.ptr, sc->flat_cid.ptr, sc->flat_progress.ptr, stream));
     // exact re-scoring with the search path's distance code: prepared queries as for a search
-    const uint32_t qstride = uint32_t(round_up(ix->dim, 16));
-    CUDA_TRY(sc->q_f32.ensure(nq * qstride));
-    CUDA_TRY(sc->q_codes.ensure(nq * qstride));
-    CUDA_TRY(sc->q_aux.ensure(nq * 2));
-    cudaError_t err = qdtype == SVSB200_F32
-        ? launch_prepare<SVSB200_F32>(d_queries, uint32_t(nq), dim, qstride, PREP_FLOAT, ix->metric, ix->dtype, ix->scale, ix->bias,
-                                      rep->d_mean, sc->q_f32.ptr, sc->q_codes.ptr, sc->q_aux.ptr, stream)
-        : launch_prepare<SVSB200_F16>(d_queries, uint32_t(nq), dim, qstride, PREP_FLOAT, ix->metric, ix->dtype, ix->scale, ix->bias,
-                                      rep->d_mean, sc->q_f32.ptr, sc->q_codes.ptr, sc->q_aux.ptr, stream);
-    CUDA_TRY(err);
+    if (int rc = prepare_queries(ix, rep, sc, d_queries, qdtype, nq, PREP_FLOAT, stream)) return rc;
     SearchParams p{};
-    p.vectors = rep->d_vectors;
+    p.vectors = rep->d_vectors.ptr;
     p.n = n;
     p.dim = dim;
     p.row_stride = ix->row_stride;
@@ -1924,14 +1773,14 @@ static int flat_on_device(svsb200_index* ix, Replica* rep, Scratch* sc, const vo
     p.scale = 1.f;
     p.qf = sc->q_f32.ptr;
     p.qaux = sc->q_aux.ptr;
-    p.qstride = qstride;
+    p.qstride = qstride_for(dim);
     p.nq = uint32_t(nq);
     p.k = uint32_t(k);
     CUDA_TRY(cudaMemsetAsync(sc->flat_unv.ptr, 0, 4, stream));
     // rounding terms of E(q) (flat.cu header): the query is always rounded to fp16, float32 data too
     p.scale = (qdtype == SVSB200_F32 ? 1.0f : 0.0f) + (ix->dtype == SVSB200_F32 ? 1.0f : 0.0f);   // number of rounded operands
     CUDA_TRY(flat_rescore(ix->dtype, l2 ? OP_L2F : OP_IPF, p, sc->flat_ckey.ptr, sc->flat_cid.ptr, nsplit, uint32_t(nq), uint32_t(k),
-                          sc->flat_qnorm.ptr, rep->flat_xmax, d_out_ids, d_out_dists, sc->flat_unv.ptr + 1, sc->flat_unv.ptr, stream));
+                          sc->flat_qnorm.ptr, rep->flat_xmax.ptr, d_out_ids, d_out_dists, sc->flat_unv.ptr + 1, sc->flat_unv.ptr, stream));
     // queries whose bound did not verify: exact scan, results scattered over the rescored rows
     uint32_t nunv = 0;
     CUDA_TRY(cudaMemcpyAsync(&nunv, sc->flat_unv.ptr, 4, cudaMemcpyDeviceToHost, stream));
@@ -1956,13 +1805,9 @@ int svsb200_flat_search_device(svsb200_index* ix, const void* d_queries, int qdt
     if (nq && (!d_queries || !d_out_ids || !d_out_dists)) return fail("svsb200_flat_search_device: NULL buffer");
     if (k == 0 || k > 1024) return fail("svsb200_flat_search_device: k must be in [1, 1024]");
     if (qdtype < SVSB200_F32 || qdtype > SVSB200_U8) return fail("bad query dtype");
-    if (ix->reps.size() != 1) return fail("svsb200_flat_search_device: the index must live on exactly one device");
-    Replica* rep = ix->reps[0].get();
-    CUDA_TRY(cudaSetDevice(rep->device));
-    std::string err;
-    Scratch* sc = scratch_for_stream(rep, static_cast<cudaStream_t>(stream_), &err);
-    if (!sc) return fail(err);
-    return flat_on_device(ix, rep, sc, d_queries, qdtype, nq, k, d_out_ids, d_out_dists, fallback_queries);
+    Scratch* sc = nullptr;
+    if (int rc = device_api_scratch("svsb200_flat_search_device", ix, stream_, &sc)) return rc;
+    return flat_on_device(ix, ix->reps[0].get(), sc, d_queries, qdtype, nq, k, d_out_ids, d_out_dists, fallback_queries);
 }
 
 int svsb200_flat_search(svsb200_index* ix, const void* queries, int qdtype, size_t nq, size_t k, uint64_t* out_ids,
@@ -1973,27 +1818,21 @@ int svsb200_flat_search(svsb200_index* ix, const void* queries, int qdtype, size
     if (k == 0 || k > 1024) return fail("svsb200_flat_search: k must be in [1, 1024]");
     if (qdtype < SVSB200_F32 || qdtype > SVSB200_U8) return fail("bad query dtype");
     Replica* rep = ix->reps[0].get();
-    CUDA_TRY(cudaSetDevice(rep->device));
-    std::string err;
-    Scratch* sc = acquire(rep, &err);
-    if (!sc) return fail(err);
-    auto body = [&]() -> int {
-        const size_t qbytes = nq * ix->dim * esize(qdtype);
-        CUDA_TRY(sc->q_raw.ensure(qbytes));
-        CUDA_TRY(sc->ids.ensure(nq * k * 8));
-        CUDA_TRY(sc->dists.ensure(nq * k));
-        CUDA_TRY(cudaMemcpyAsync(sc->q_raw.ptr, queries, qbytes, cudaMemcpyHostToDevice, sc->stream));
-        int rc = flat_on_device(ix, rep, sc, sc->q_raw.ptr, qdtype, nq, k, reinterpret_cast<uint64_t*>(sc->ids.ptr), sc->dists.ptr,
-                                nullptr);
-        if (rc) return rc;
-        CUDA_TRY(cudaMemcpyAsync(out_ids, sc->ids.ptr, nq * k * 8, cudaMemcpyDeviceToHost, sc->stream));
-        CUDA_TRY(cudaMemcpyAsync(out_dists, sc->dists.ptr, nq * k * 4, cudaMemcpyDeviceToHost, sc->stream));
-        CUDA_TRY(cudaStreamSynchronize(sc->stream));
-        return 0;
-    };
-    int rc = body();
-    release(rep, sc);
-    return rc;
+    ScratchLease lease;
+    if (int rc = lease.take(rep, nullptr)) return rc;
+    Scratch* sc = lease.sc;
+    const size_t qbytes = nq * ix->dim * esize(qdtype);
+    CUDA_TRY(sc->q_raw.ensure(qbytes));
+    CUDA_TRY(sc->ids.ensure(nq * k * 8));
+    CUDA_TRY(sc->dists.ensure(nq * k));
+    CUDA_TRY(cudaMemcpyAsync(sc->q_raw.ptr, queries, qbytes, cudaMemcpyHostToDevice, sc->stream));
+    int rc = flat_on_device(ix, rep, sc, sc->q_raw.ptr, qdtype, nq, k, reinterpret_cast<uint64_t*>(sc->ids.ptr), sc->dists.ptr,
+                            nullptr);
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(out_ids, sc->ids.ptr, nq * k * 8, cudaMemcpyDeviceToHost, sc->stream));
+    CUDA_TRY(cudaMemcpyAsync(out_dists, sc->dists.ptr, nq * k * 4, cudaMemcpyDeviceToHost, sc->stream));
+    CUDA_TRY(cudaStreamSynchronize(sc->stream));
+    return 0;
 }
 
 int svsb200_exhaustive_device(svsb200_index* ix, const void* d_queries, int qdtype, size_t nq, size_t k, uint64_t* d_out_ids,
@@ -2001,13 +1840,9 @@ int svsb200_exhaustive_device(svsb200_index* ix, const void* d_queries, int qdty
     if (!ix) return fail("svsb200_exhaustive_device: NULL index");
     if (nq && (!d_queries || !d_out_ids || !d_out_dists)) return fail("svsb200_exhaustive_device: NULL buffer");
     if (k == 0 || k > 1024) return fail("svsb200_exhaustive_device: k must be in [1, 1024]");
-    if (ix->reps.size() != 1) return fail("svsb200_exhaustive_device: the index must live on exactly one device");
-    Replica* rep = ix->reps[0].get();
-    CUDA_TRY(cudaSetDevice(rep->device));
-    std::string err;
-    Scratch* sc = scratch_for_stream(rep, static_cast<cudaStream_t>(stream_), &err);
-    if (!sc) return fail(err);
-    return search_on_device(ix, rep, sc, d_queries, qdtype, nq, k, k, k, d_out_ids, 8, d_out_dists, sc->stream, true);
+    Scratch* sc = nullptr;
+    if (int rc = device_api_scratch("svsb200_exhaustive_device", ix, stream_, &sc)) return rc;
+    return search_on_device(ix, ix->reps[0].get(), sc, d_queries, qdtype, nq, k, k, k, d_out_ids, 8, d_out_dists, sc->stream, true);
 }
 
 }  // extern "C"
